@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- flux cell-updates/s of the fused per-cell flux chain (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload C4|C2|C3|C5] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload C4|C2|C3|C5] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one coupling step (early + normal phase fused: fc_step_all) over the synthetic exchange grid.
 Default workload C4 = BASELINE.json configs[3], the configuration the metric's roofline target is quoted on:
@@ -21,6 +21,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -141,17 +142,47 @@ def build_scenario(workload, offset_size=None, cells=None):
     return sc
 
 
+DUMP_BYTES = 48 << 20      # --dump-outputs: all files together stay below 64 MB
+DUMP_SEED = 20240601
+
+
+def dump_outputs(out_dir, fields, n_total, off, diag_sums, dist, rank, world):
+    """what the timed path computed in its last step, written by rank 0: every output field as type<i>_grid<g>_<name>.npy
+    (float64, in global cell order) and, with diagnostics, their area-weighted sums in the same (sorted) field order as
+    diagnostics_sum.npy.  When the whole grids would exceed DUMP_BYTES, every field holds the same fixed, seeded sample of
+    global cells, so two builds run with the same arguments can be compared value for value."""
+    keys = sorted(fields)
+    m = min(n_total, DUMP_BYTES // (8 * len(keys)))
+    cells = np.arange(n_total) if m == n_total else np.sort(np.random.default_rng(DUMP_SEED).choice(n_total, m, replace=False))
+    mine = cells[(cells >= off) & (cells < off + fields[keys[0]].n)] - off
+    local = {k: fields[k].download()[mine] for k in keys}
+    parts = [local]
+    if dist:
+        parts = [None] * world if rank == 0 else None
+        dist.gather_object(local, parts, dst=0)      # the shards are contiguous ranges in rank order
+    if rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        for k in keys:
+            np.save(os.path.join(out_dir, "type%d_grid%d_%s.npy" % k), np.concatenate([p[k] for p in parts]))
+        if diag_sums is not None:
+            np.save(os.path.join(out_dir, "diagnostics_sum.npy"), np.asarray(diag_sums, dtype=np.float64))
+
+
+_native_dir = None      # the host-specific oracle builds: a temporary directory, the tree may be read-only
+
+
 def native_oracle(build="fast"):
     """the oracle built for THIS host: 'fast' = -O3 -march=native -ffast-math (the reference's release flags, -O3 -fp-model fast=2
     -xHost, build_hlrng.sh:26), 'parity' = -O2 -ffp-contract=off (its debug / -fp-model precise build, :23); falls back to
     the shipped builds"""
+    global _native_dir
     import ctypes as C
     from oracle_py import ORACLE_DIR
     flags = {"fast": ["-O3", "-march=native", "-ffast-math"], "parity": ["-O2", "-march=native", "-ffp-contract=off"]}[build]
-    out = os.path.join(ORACLE_DIR, "_native")
     try:
-        os.makedirs(out, exist_ok=True)
-        so = os.path.join(out, "liboracle_%s.so" % build)
+        if _native_dir is None:
+            _native_dir = tempfile.TemporaryDirectory(prefix="fluxcalc_oracle_")
+        so = os.path.join(_native_dir.name, "liboracle_%s.so" % build)
         subprocess.check_call(["gcc", "-std=c11"] + flags + ["-fPIC", "-shared", "-o", so,
                                os.path.join(ORACLE_DIR, "flux_oracle.c"), os.path.join(ORACLE_DIR, "cpu_baseline.c"),
                                "-lm", "-lpthread"], stderr=subprocess.DEVNULL)
@@ -250,9 +281,16 @@ def main():
     ap.add_argument("--comm", default="p2p", choices=["p2p", "nccl"],
                     help="N>1 diagnostics exchange: peer mailboxes written by the step's kernel over NVLink (default; falls back "
                          "to NCCL when CUDA IPC is unavailable) or ncclAllReduce on a side stream")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float64; a fixed, seeded sample of the cells "
+                         "when the whole grids would exceed 48 MiB) to compare two builds")
     args = ap.parse_args()
     if args.steps is None:
         args.steps = 1000 if (args.workload == "C5" and args.impl == "b200") else 200
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -374,6 +412,9 @@ def main():
     clocks = sampler.stop()
     graph_launches = fc.info("graph_launches")
     launches = fc.info("launches") - launches0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {k: wrapped[id(a)] for k, a in g_out.items()}, n_total, off,
+                     [fc.diagnostics(*k)[0] for k in sorted(g_out)] if diag else None, dist, rank, world)
     # kernel time for the roofline: the SAME step loop continued right after the timed region, every n-th launch between an
     # event pair.  Not inside the timed region: an event between two launches switches their programmatic overlap, the early
     # ring fill and the per-CTA hand-over off, which costs 7-18 us per bracketed launch on an 8-GPU shard (call 14: three
