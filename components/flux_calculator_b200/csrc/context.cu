@@ -575,7 +575,6 @@ extern "C" int fc_set_option(fc_context *c, const char *name, int64_t value)
     else if (!strcmp(name, "diagnostics")) c->diagnostics = (int)std::max<int64_t>(0, std::min<int64_t>(value, 2));
     else if (!strcmp(name, "staged")) c->use_staged = (int)std::max<int64_t>(0, std::min<int64_t>(value, 2));
     else if (!strcmp(name, "early_loads")) c->early_loads = value != 0;
-    else if (!strcmp(name, "graphs")) c->use_graphs = value != 0;
     else if (!strcmp(name, "chain")) c->chain_steps = value != 0;
     else if (!strcmp(name, "download")) c->download_sent_only = value != 0;
     else if (!strcmp(name, "dyn_min_tiles")) c->dyn_min_tiles = (int)std::max<int64_t>(0, std::min<int64_t>(value, 1 << 30));
@@ -583,7 +582,6 @@ extern "C" int fc_set_option(fc_context *c, const char *name, int64_t value)
         c->tail_own_step = false;
         return FC_OK;
     }
-    else if (!strcmp(name, "prefetch_distance")) c->prefetch_distance = (int)std::max<int64_t>(0, std::min<int64_t>(value, 1 << 20));
     else if (!strcmp(name, "profile_kernel")) {
         c->profile_kernel = (int)std::max<int64_t>(0, std::min<int64_t>(value, 1 << 20));   // 0 off, n: every n-th launch
         c->prof_seq = 0;
@@ -1215,7 +1213,6 @@ static bool build_fused(fc_context *c, bool do_early, bool do_normal, FusedBundl
     // diagnostics slots
     P.diag = 0;
     memset(P.diag_map, 0xff, sizeof P.diag_map);
-    P.prefetch_distance = c->prefetch_distance;
     if (c->diagnostics) {
         for (int g = 1; g <= 3; ++g)
             if ((g == 1 || do_normal) && !c->area_dev[g] && c->n[g] > 0) return false;   // reported by prepare
@@ -1875,14 +1872,14 @@ extern "C" int fc_run_steps(fc_context *c, int64_t t0, int64_t dt, int nsteps)
             for (int b : {h.out, h.in[0], h.in[1]})
                 if (b >= 0) resident = resident && c->bufs[b].user_is_device;
     }
-    const bool use_graphs = resident && c->use_graphs && !c->profile_kernel;
+    const bool graphs = resident && !c->profile_kernel;
     int k = 0;
     while (k < nsteps) {
         const int64_t t = t0 + (int64_t)k * dt;
         const int month = F.ok && F.plan.t.bias ? fc_current_month(c->init_date, t) : 1;
         int run = 1;      // steps k .. k + run - 1 share the month
         while (k + run < nsteps && (!(F.ok && F.plan.t.bias) || fc_current_month(c->init_date, t0 + (int64_t)(k + run) * dt) == month)) ++run;
-        while (use_graphs && run >= kGraphSteps) {
+        while (graphs && run >= kGraphSteps) {
             cudaGraphExec_t &g = c->step_graph[month];
             if (!g)
                 if (int rc = capture_steps(c, F, month, kGraphSteps, &g)) return rc;

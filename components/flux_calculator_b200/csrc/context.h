@@ -148,7 +148,6 @@ struct fc_context {
     int diagnostics = 0;         // 0 off, 1 area-weighted sums, 2 sums + min/max
     int h2d_chunks = 0;          // 0 = auto
     int use_staged = 1;          // specialised persistent kernel (spec_kernel.cu): 0 never, >= 1 whenever the plan fits
-    int prefetch_distance = 0;   // L2 prefetch look-ahead of the fused kernel, in 512-cell blocks (0 = off)
 
     // derived
     bool dirty = true;
@@ -217,7 +216,6 @@ struct fc_context {
 
     // fc_run_steps: one instantiated graph of kGraphSteps step launches per calendar month (index 1..12)
     cudaGraphExec_t step_graph[13] = {};
-    bool use_graphs = true;
     bool download_sent_only = false;        // option "download" = 1: only registered output fields travel back to the host
     int dyn_min_tiles = 0;                  // option: tiles per CTA from which the specialised kernel schedules dynamically (0: default)
     int64_t graph_launches = 0;

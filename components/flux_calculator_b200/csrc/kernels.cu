@@ -415,65 +415,6 @@ __device__ __forceinline__ bool uv_chain(const FusedPlan &p, const FusedUV &g, i
     return bad;
 }
 
-// L2 prefetch of the tile a later CTA will work on: one bulk prefetch per input array, issued by one thread.
-// It needs no register or scoreboard slot, so DRAM latency is paid ahead of time and the demand loads of
-// CTA b+distance hit L2 (ncu: long_scoreboard was the dominant stall at 14-16 resident warps/SM).
-__device__ __forceinline__ void prefetch_l2(const double *p, int64_t cell, int64_t end)
-{
-    if (p == nullptr || cell >= end) return;
-    const int64_t n = (end - cell) < kFusedCellsPerBlock ? (end - cell) : kFusedCellsPerBlock;
-    const uint32_t bytes = (uint32_t)(n * 8) & ~15u;
-    if (bytes)
-        asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(p + cell), "r"(bytes) : "memory");
-}
-
-__device__ __forceinline__ void prefetch_tile(const FusedPlan &p, int which, int64_t cell, int64_t end)
-{
-    if (which == 0) {
-        const FusedT &t = p.t;
-        if (p.do_normal) {
-            prefetch_l2(t.bias, cell, end);
-            prefetch_l2(t.rsdd, cell, end);
-        }
-        prefetch_l2(t.area, cell, end);
-        const double *last[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-        for (int i = 0; i < p.S; ++i) {
-            const FusedTType &ty = t.ty[i];
-            const double *q[8] = {ty.psur, ty.qatm, ty.tatm, ty.patm, ty.uatm, ty.vatm, ty.a_evap, ty.a_sens};
-#pragma unroll
-            for (int k = 0; k < 8; ++k)
-                if (q[k] != last[k]) {      // atmosphere fields are shared by the surface types
-                    last[k] = q[k];
-                    if (p.do_normal) prefetch_l2(q[k], cell, end);
-                }
-            prefetch_l2(ty.tsur, cell, end);
-            prefetch_l2(ty.fare, cell, end);
-            if (p.do_normal) {
-                prefetch_l2(ty.fice, cell, end);
-                prefetch_l2(ty.qsur_in, cell, end);
-            }
-        }
-    } else {
-        const FusedUV &g = p.uv[which - 1];
-        prefetch_l2(g.area, cell, end);
-        const double *last[4] = {nullptr, nullptr, nullptr, nullptr};
-        for (int i = 0; i < p.S; ++i) {
-            const FusedUVType &ty = g.ty[i];
-            const double *q[4] = {ty.psur, ty.uatm, ty.vatm, ty.a_mom};
-#pragma unroll
-            for (int k = 0; k < 4; ++k)
-                if (q[k] != last[k]) {
-                    last[k] = q[k];
-                    prefetch_l2(q[k], cell, end);
-                }
-            prefetch_l2(ty.fice, cell, end);
-            prefetch_l2(ty.tsur, cell, end);
-            prefetch_l2(ty.fare, cell, end);
-            prefetch_l2(ty.qsur_in, cell, end);
-        }
-    }
-}
-
 // FULL = true : every thread owns V whole cells and every array is 16-byte aligned (128-bit accesses only);
 //               launched over floor(cells/V) cell vectors per grid.
 // FULL = false: guarded scalar accesses; launched over the ragged remainder (cells % V) of each grid, or over
@@ -483,7 +424,6 @@ struct LaunchGeom {
     int64_t first[3];        // first cell handled by this launch on each grid
     int64_t count[3];        // cells handled by this launch on each grid
     int64_t row0;            // first diagnostics row of this launch
-    int prefetch_distance;   // in blocks, 0 = off
 };
 
 // cold, out of line: every lane of the warp that called recomputes its V cells with the IEEE policy (identical bits for the
@@ -521,8 +461,6 @@ fused_step_kernel(const __grid_constant__ FusedPlan p, const __grid_constant__ L
     const int64_t end = geo.first[which] + geo.count[which];
     const int64_t j = geo.first[which] + ((int64_t)blk * kFusedThreads + threadIdx.x) * V;
     const int nv = (j >= end) ? 0 : (end - j >= V ? V : (int)(end - j));
-    if (FULL && geo.prefetch_distance > 0 && threadIdx.x == 0)
-        prefetch_tile(p, which, geo.first[which] + (int64_t)(blk + geo.prefetch_distance) * kFusedCellsPerBlock, end);
     DiagCtx dg;
     if (DIAG) {
         dg.base = p.diag_partials;
@@ -791,8 +729,6 @@ static FusedGeom fused_geometry(const FusedPlan &p)
     G.nb_tail = nbt[0] + nbt[1] + nbt[2];
     G.main.row0 = 0;
     G.tail.row0 = (int64_t)G.nb_main * (kFusedThreads / 32);
-    G.main.prefetch_distance = p.prefetch_distance;
-    G.tail.prefetch_distance = 0;
     // specialised persistent kernel for the canonical plans with one or two surface types, whatever the grid size (20 000 cells:
     // 6 us per step against 20 us on the generic kernels); it takes the ragged remainder along: one launch
     G.spec = false;

@@ -172,7 +172,6 @@ struct FusedPlan {
     double *diag_partials;   // [plane: sum|min|max][diag_n][diag_rows]
     int64_t diag_rows;       // warp rows of one fused step (row stride of the partials)
     int diag_n;              // number of active diagnostics slots
-    int prefetch_distance;   // L2 prefetch look-ahead in blocks (0 = off)
     signed char diag_map[(kMaxSurfaceTypes + 1) * 10];   // slot -> compact index, -1 = inactive
     int staged;              // specialised persistent kernel: 0 never, >= 1 whenever the plan fits
     int pad2;
@@ -184,10 +183,7 @@ constexpr int kDiagSlots = (kMaxSurfaceTypes + 1) * DQ_COUNT;
 static_assert(kDiagSlots == kDiagSlotsFwd, "DiagMail layout");
 
 constexpr int kFusedThreads = 256;
-#ifndef FC_MIN_BLOCKS
-#define FC_MIN_BLOCKS 2
-#endif
-constexpr int kFusedMinBlocks = FC_MIN_BLOCKS;               // __launch_bounds__ occupancy target
+constexpr int kFusedMinBlocks = 2;                           // __launch_bounds__ occupancy target
 constexpr int kFusedVec = 2;                                  // cells per thread (128-bit accesses)
 constexpr int kFusedCellsPerBlock = kFusedThreads * kFusedVec;
 

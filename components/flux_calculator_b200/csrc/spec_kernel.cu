@@ -37,7 +37,6 @@
 
 #include <cuda_runtime.h>
 #include <float.h>
-#include <stdlib.h>
 #include <string.h>
 
 namespace fc {
@@ -45,37 +44,21 @@ namespace fc {
 constexpr int kSpecV = 2;
 // CTA geometry per number of surface types.  One type: 2 CTAs per SM, one team of 8 consumer warps, 512-cell tiles.
 // Two types (15-16 input arrays per t tile): 1 CTA per SM, two teams of 8 warps sharing three 60 KB t stages (two in
-// work, one in flight); the finer variant (four teams of 4 warps on 256-cell tiles, 7 stages of 30 KB) measured slower.
-// Tuning switches, settled by an A/B on one B200 (profiles/run18.sh, 3 repetitions each, C5 = 10^7 cells, two types):
+// work, one in flight).  Lane 0 of the producer warp issues all bulk copies of a tile.  Measured on one B200
+// (profiles/run18.sh, 3 repetitions each, C5 = 10^7 cells, two types) against four teams of 4 warps on 256-cell tiles
+// (7 stages of 30 KB) and against a producer in which lane a issues the copy of slot a:
 //   teams x producer          2 x one lane   2 x lane per slot   4 x one lane   4 x lane per slot
 //   C5 ms / step              0.852-0.861    0.892-0.905         1.054-1.058    0.898-0.906
 //   C4 ms / step (one type)   0.434-0.445    0.437               0.435-0.444    0.437
-#ifndef FC_SPEC2_TEAMS
-#define FC_SPEC2_TEAMS 2            // two surface types: 2 teams x 8 warps x 512-cell tiles, or 4 teams x 4 warps x 256-cell tiles
-#endif
-#ifndef FC_SPEC2_TEAM_WARPS
-#define FC_SPEC2_TEAM_WARPS (16 / FC_SPEC2_TEAMS)
-#endif
-#ifndef FC_SPEC2_REGS
-#define FC_SPEC2_REGS 96            // two types: 17 warps.  One of the four SM sub-partitions (16384 registers each) holds five of them:
-#endif                              // 5 x 32 x 96 fits, 5 x 32 x 104 does not ("too many resources requested for launch" at 112 and 120)
-#ifndef FC_SPEC1_REGS
-#define FC_SPEC1_REGS 96            // one type: 2 CTAs x 9 warps per SM (112 would still fit the register file on paper, but measured
-                                    // 0.57 ms instead of 0.43 ms on C4: the second CTA no longer becomes resident)
-#endif
-#ifndef FC_SPEC_BYPASS
-#define FC_SPEC_BYPASS 0            // bit (NS - 1) set: in the kernels for NS surface types the two t-grid arrays that are used exactly once per surface
-#endif                              // type and feed no transcendental -- RSDD (copied through) and the evaporation bias (added) -- do NOT travel through
-                                    // the ring: each consumer thread fetches its own 16 bytes of them straight from global memory before it waits for
-                                    // the tile.  Two types: the t stage shrinks from 15 to 13 arrays (60 -> 52 KB), which buys a FOURTH stage (two in
-                                    // work, two in flight instead of one); one type: 11 -> 9 arrays, three stages per CTA instead of two.
-#ifndef FC_SPEC_PAR_PRODUCER
-#define FC_SPEC_PAR_PRODUCER 0      // 0: lane 0 of the producer warp issues all bulk copies of a tile; 1: lane a issues slot a
-#endif
+// Registers per thread, 96 for both:
+//   one type: 2 CTAs x 9 warps per SM (112 would still fit the register file on paper, but measured 0.57 ms instead of
+//   0.43 ms on C4: the second CTA no longer becomes resident);
+//   two types: 17 warps.  One of the four SM sub-partitions (16384 registers each) holds five of them: 5 x 32 x 96 fits,
+//   5 x 32 x 104 does not ("too many resources requested for launch" at 112 and 120).
 template <int NS>
 struct SpecGeom {
-    static constexpr int kTeams = (NS == 1) ? 1 : FC_SPEC2_TEAMS;
-    static constexpr int kTeamWarps = (NS == 1) ? 8 : FC_SPEC2_TEAM_WARPS;     // consumer warps of one team = one tile per pass
+    static constexpr int kTeams = (NS == 1) ? 1 : 2;
+    static constexpr int kTeamWarps = 8;                     // consumer warps of one team = one tile per pass
     static constexpr int kTeamThreads = kTeamWarps * 32;
     static constexpr int kTile = kTeamThreads * kSpecV;      // cells per tile
     static constexpr int kSlotBytes = kTile * 8;             // one array of one tile
@@ -83,11 +66,8 @@ struct SpecGeom {
     static constexpr int kThreads = kConsumers + 32;         // + producer warp
     static constexpr int kWarps = kTeams * kTeamWarps;
     static constexpr int kCtasPerSm = (NS == 1) ? 2 : 1;
-    // registers per thread, stated directly (see the two macros above)
-    static constexpr int kMaxRegs = (NS == 1) ? FC_SPEC1_REGS : FC_SPEC2_REGS;
+    static constexpr int kMaxRegs = 96;                      // registers per thread (see above)
 };
-template <int NS>
-constexpr bool kSpecBypass = ((FC_SPEC_BYPASS >> (NS - 1)) & 1) != 0;
 constexpr int kSpecMaxStages = 16;
 constexpr int kSpecMaxBars = 32;                         // barriers per set: lcm(teams, stages) <= 2 * 16
 constexpr int kSpecMaxSlots = 16;
@@ -105,18 +85,15 @@ enum SpecSet { SET_BULK = 0, SET_RCO = 1 };
 template <int SET, int NS>
 struct Lay {
     static constexpr int kPer = (NS == 1) ? 2 : 3;       // per-type arrays: FICE, TSUR (, FARE)
-    // t grid.  With FC_SPEC_BYPASS for this NS, RSDD and BIAS move behind the staged slots (they do not travel through the ring)
-    static constexpr bool kBy = kSpecBypass<NS>;
-    static constexpr int PSUR = 0, QATM = 1, TATM = 2, UATM = 3, VATM = 4;
-    static constexpr int AEV = kBy ? 5 : 7, PATM = kBy ? 6 : 8;      // bulk only
-    static constexpr int kShared = (SET == SET_BULK ? 7 : 5) + (kBy ? 0 : 2);
+    // t grid
+    static constexpr int PSUR = 0, QATM = 1, TATM = 2, UATM = 3, VATM = 4, RSDD = 5, BIAS = 6;
+    static constexpr int AEV = 7, PATM = 8;              // bulk only
+    static constexpr int kShared = (SET == SET_BULK) ? 9 : 7;
     __host__ __device__ static constexpr int FICE(int i) { return kShared + kPer * i; }
     __host__ __device__ static constexpr int TSUR(int i) { return kShared + kPer * i + 1; }
     __host__ __device__ static constexpr int FARE(int i) { return kShared + kPer * i + 2; }
     static constexpr int ASE = kShared + kPer * NS;      // bulk/MOM5 only (CHEA != CMOI)
-    static constexpr int kStagedT = ASE + (SET == SET_BULK ? 1 : 0);      // t slots [0, kStagedT) travel through the ring
-    static constexpr int RSDD = kBy ? kStagedT : 5, BIAS = kBy ? kStagedT + 1 : 6;
-    static constexpr int NT = kStagedT + (kBy ? 2 : 0);
+    static constexpr int NT = ASE + (SET == SET_BULK ? 1 : 0);
     // u / v grid
     static constexpr int U_UATM = 0, U_VATM = 1, U_PSUR = 2, U_AMOM = 3;
     static constexpr int kUShared = (SET == SET_BULK) ? 4 : 2;
@@ -133,7 +110,7 @@ struct SpecPlan {
     int64_t end[3];                   // one past its last cell
     int ntiles[3];                    // ceil(cells / tile): the last tile of a grid may be partial (guarded path)
     int rot[3];                       // static schedule: CTA that takes tile 0 of each grid
-    int t_staged;                     // t slots [0, t_staged) travel through the ring (FC_SPEC_BYPASS: the last two do not)
+    int ns;                           // number of surface types (the kernel has it as NS)
     int t_stages, u_stages;           // the two carvings of the ring
     int t_stage_bytes, u_stage_bytes;
     int t_bars, u_bars;               // lcm(teams, stages): tile i uses barrier i mod bars (one per (team, stage) pair) in phase i / bars
@@ -142,7 +119,6 @@ struct SpecPlan {
     int any_avg_t;                    // some t-grid flux is area-fraction averaged (FARE is staged)
     int ase_slot;                     // bulk: slot of the sensible-heat transfer coefficient (AEV for CCLM, ASE for MOM5)
     int diag;
-    int ns;
     double latent_heat[kSpecMaxNS];
     const double *src[3][kSpecMaxSlots];   // per grid: source array of each stage slot (null: slot unused)
     uint32_t tx_bytes[3];             // bytes one tile of that grid brings in
@@ -220,22 +196,6 @@ struct LdStage {
     const char *base;
     __device__ __forceinline__ S2 operator()(int slot) const
     {
-        const double2 t = *reinterpret_cast<const double2 *>(base + slot * SLOT_BYTES);
-        S2 r;
-        r.v[0] = t.x;
-        r.v[1] = t.y;
-        return r;
-    }
-};
-// hot path with FC_SPEC_BYPASS: the same, except that RSDD and BIAS come from registers (fetched by spec_fetch_direct)
-template <int SLOT_BYTES, int RSDD, int BIAS>
-struct LdStageDirect {
-    const char *base;
-    S2 rsdd, bias;
-    __device__ __forceinline__ S2 operator()(int slot) const
-    {
-        if (slot == RSDD) return rsdd;
-        if (slot == BIAS) return bias;
         const double2 t = *reinterpret_cast<const double2 *>(base + slot * SLOT_BYTES);
         S2 r;
         r.v[0] = t.x;
@@ -665,37 +625,6 @@ __device__ __forceinline__ void spec_uv_chain(M &m, const SpecPlan &p, int north
     }
 }
 
-// FC_SPEC_BYPASS: this thread's 16 bytes of the two t-grid arrays that do not travel through the ring.  Issued before the
-// thread waits for its tile (static schedule: the cells are known in advance) or right after (dynamic schedule); first
-// used a good way into the chain (the bias after the first QSUR and MEVA, RSDD at the end of the first surface type).
-template <int SET, int NS>
-__device__ __forceinline__ void spec_fetch_direct(const SpecPlan &p, int64_t j, S2 &rsdd, S2 &bias)
-{
-    using L = Lay<SET, NS>;
-    double2 r = make_double2(0.0, 0.0), b = make_double2(0.0, 0.0);
-    if (p.has_rsdr) r = __ldg(reinterpret_cast<const double2 *>(p.src[0][L::RSDD] + j));
-    if (p.has_bias) b = __ldg(reinterpret_cast<const double2 *>(p.src[0][L::BIAS] + j));
-    rsdd.v[0] = r.x;
-    rsdd.v[1] = r.y;
-    bias.v[0] = b.x;
-    bias.v[1] = b.y;
-}
-
-// the t chain of one full tile out of a ring stage
-template <int SET, int NS, class ST, class DG>
-__device__ __forceinline__ void spec_t_tile(FastVec<kSpecV> &m, const SpecPlan &p, const char *base, const S2 &rsdd, const S2 &bias,
-                                            const ST &st, DG &dg)
-{
-    using L = Lay<SET, NS>;
-    if constexpr (kSpecBypass<NS>) {
-        const LdStageDirect<SpecGeom<NS>::kSlotBytes, L::RSDD, L::BIAS> ld{base, rsdd, bias};
-        spec_t_chain<SET, NS>(m, p, ld, st, dg);
-    } else {
-        const LdStage<SpecGeom<NS>::kSlotBytes> ld{base};
-        spec_t_chain<SET, NS>(m, p, ld, st, dg);
-    }
-}
-
 // ---------------------------------------------------------------------------------------------
 // cold epilogue of one phase of one warp: recompute the flagged tiles with the IEEE routines (scalar, from global
 // memory), then rebuild this warp's diagnostics of the phase from the stored outputs in the hot loop's order:
@@ -772,9 +701,6 @@ __device__ __noinline__ void spec_cold_phase(const SpecPlan &p, int ph, int64_t 
 // makes exactly two failing claims (two are kept in flight), so a launch advances it by (units + 2 CTAs) and the host
 // keeps the base.  Small grids (few tiles per CTA: nothing to balance, and the claims' latency shows) and launches
 // with diagnostics (the per-thread running sums need a reproducible tile -> thread map) use the static schedule.
-#ifndef FC_SPEC_DYNAMIC
-#define FC_SPEC_DYNAMIC 1
-#endif
 constexpr int kDynPartial = 1 << 30;      // tile id flag: partial tile, nothing in the stage
 constexpr unsigned kDynUvBatch = 4;       // u/v tiles per claim
 
@@ -844,7 +770,7 @@ __device__ __forceinline__ void spec_dynamic_body(const SpecPlan &p, char *ring,
                     mbar_expect_tx(&fullT[bi], p.tx_bytes[0]);
                     char *dst = ring + (size_t)st * p.t_stage_bytes;
 #pragma unroll 1
-                    for (int a = 0; a < L::kStagedT; ++a)
+                    for (int a = 0; a < L::NT; ++a)
                         if (p.src[0][a]) bulk_g2s(dst + a * GEO::kSlotBytes, p.src[0][a] + cell, GEO::kSlotBytes, &fullT[bi]);
                 }
                 next();
@@ -955,9 +881,8 @@ __device__ __forceinline__ void spec_dynamic_body(const SpecPlan &p, char *ring,
                     const LdStage<GEO::kSlotBytes> ld{ring + (size_t)s * sbytes + toff};
                     spec_uv_chain<SET, NS>(m, p, north, ld, st, nd);
                 } else {
-                    S2 d_rsdd, d_bias;
-                    if constexpr (kSpecBypass<NS>) spec_fetch_direct<SET, NS>(p, j, d_rsdd, d_bias);
-                    spec_t_tile<SET, NS>(m, p, ring + (size_t)s * sbytes + toff, d_rsdd, d_bias, st, nd);
+                    const LdStage<GEO::kSlotBytes> ld{ring + (size_t)s * sbytes + toff};
+                    spec_t_chain<SET, NS>(m, p, ld, st, nd);
                 }
                 bad = m.bad();
             } else {
@@ -1110,7 +1035,7 @@ __global__ void __launch_bounds__(SpecGeom<NS>::kThreads) __maxnreg__(SpecGeom<N
                         __syncwarp();
                         for (int cs = b; cs < p.prev.nslots; cs += G) diag_fold_slot(p.prev, cs);
                     }
-                    if (!FC_SPEC_PAR_PRODUCER && lane != 0 && !(chain && b < p.prev.nslots)) return;
+                    if (lane != 0 && !(chain && b < p.prev.nslots)) return;
                 }
                 if (i >= ring0) break;
                 if (i >= NT) {
@@ -1124,13 +1049,9 @@ __global__ void __launch_bounds__(SpecGeom<NS>::kThreads) __maxnreg__(SpecGeom<N
                 if (lane == 0) mbar_expect_tx(&fullT[bi], p.tx_bytes[0]);
                 __syncwarp();
                 char *dst = ring + (size_t)st * p.t_stage_bytes;
-                static_assert(Lay<SET, NS>::NT <= 32 && Lay<SET, NS>::NUV <= 32, "one lane per slot");
-                if (FC_SPEC_PAR_PRODUCER) {
-                    if (lane < Lay<SET, NS>::kStagedT && p.src[0][lane])
-                        bulk_g2s(dst + lane * GEO::kSlotBytes, p.src[0][lane] + cell, GEO::kSlotBytes, &fullT[bi]);
-                } else if (lane == 0) {
+                if (lane == 0) {
 #pragma unroll 1
-                    for (int a = 0; a < Lay<SET, NS>::kStagedT; ++a)
+                    for (int a = 0; a < Lay<SET, NS>::NT; ++a)
                         if (p.src[0][a]) bulk_g2s(dst + a * GEO::kSlotBytes, p.src[0][a] + cell, GEO::kSlotBytes, &fullT[bi]);
                 }
                 if (++st == NT) st = 0;
@@ -1166,10 +1087,7 @@ __global__ void __launch_bounds__(SpecGeom<NS>::kThreads) __maxnreg__(SpecGeom<N
                     if (lane == 0) mbar_expect_tx(&fullU[bi], p.tx_bytes[ph]);
                     __syncwarp();
                     char *dst = ring + (size_t)st * p.u_stage_bytes;
-                    if (FC_SPEC_PAR_PRODUCER) {
-                        if (lane < Lay<SET, NS>::NUV && p.src[ph][lane])
-                            bulk_g2s(dst + lane * GEO::kSlotBytes, p.src[ph][lane] + cell, GEO::kSlotBytes, &fullU[bi]);
-                    } else if (lane == 0) {
+                    if (lane == 0) {
 #pragma unroll 1
                         for (int a = 0; a < Lay<SET, NS>::NUV; ++a)
                             if (p.src[ph][a]) bulk_g2s(dst + a * GEO::kSlotBytes, p.src[ph][a] + cell, GEO::kSlotBytes, &fullU[bi]);
@@ -1232,12 +1150,11 @@ __global__ void __launch_bounds__(SpecGeom<NS>::kThreads) __maxnreg__(SpecGeom<N
                 dg.area.v[1] = a_next.y;
                 if (p.area_ahead && i + TEAMS < ring0) a_next = __ldg(reinterpret_cast<const double2 *>(p.area[0] + j + ahead));
             }
-            S2 d_rsdd, d_bias;
-            if constexpr (kSpecBypass<NS>) spec_fetch_direct<SET, NS>(p, j, d_rsdd, d_bias);      // in flight while the thread waits for the tile
             mbar_wait(&fullT[bi], use & 1);
             FastVec<kSpecV> m;
+            const LdStage<GEO::kSlotBytes> ld{ring + (size_t)s * p.t_stage_bytes + toff};
             const StPair st{j};
-            spec_t_tile<SET, NS>(m, p, ring + (size_t)s * p.t_stage_bytes + toff, d_rsdd, d_bias, st, dg);
+            spec_t_chain<SET, NS>(m, p, ld, st, dg);
             __syncwarp();
             if (lane == 0) mbar_arrive(&emptyT[bi]);
             if (__any_sync(0xffffffffu, m.bad()) && lane == 0) {
@@ -1439,8 +1356,7 @@ static bool spec_fill(const FusedPlan &p, SpecPlan &sp)
     }
     // the two carvings of the ring: as many stages as fit (2 CTAs per SM with one type, the whole SM with two)
     int t_slots = 0, u_slots = 0;
-    sp.t_staged = L::kStagedT;
-    for (int a = 0; a < L::kStagedT; ++a)
+    for (int a = 0; a < L::NT; ++a)
         if (sp.src[0][a]) t_slots = a + 1;
     for (int g = 1; g < 3; ++g)
         for (int a = 0; a < L::NUV; ++a)
@@ -1537,7 +1453,7 @@ static bool spec_build(const FusedPlan &p, const int64_t first[3], const int64_t
     if (!ok) return false;
     for (int g = 0; g < 3; ++g) {
         int n = 0;
-        for (int k = 0; k < (g == 0 ? sp.t_staged : kSpecMaxSlots); ++k) n += sp.src[g][k] != nullptr;
+        for (int k = 0; k < kSpecMaxSlots; ++k) n += sp.src[g][k] != nullptr;
         sp.tx_bytes[g] = (uint32_t)n * (uint32_t)((p.S == 1) ? SpecGeom<1>::kSlotBytes : SpecGeom<2>::kSlotBytes);
     }
     sp.area[0] = t.area;
@@ -1584,17 +1500,15 @@ int spec_applicable(const FusedPlan &p, const int64_t first[3], const int64_t ce
 // producer makes one failing claim); 0: the plan runs on the static schedule
 // tiles per CTA from which the dynamic schedule is used: below, the static one has nothing to lose to imbalance and the
 // claims would only add latency (measured, RCO set at 10^6 cells = 20 tiles per CTA: 29.2 us static, 32.7 us dynamic)
-#ifndef FC_SPEC_DYN_MIN_TILES
-#define FC_SPEC_DYN_MIN_TILES 48
-#endif
+constexpr int kSpecDynMinTiles = 48;
 static bool spec_wants_dyn(const SpecPlan &sp)
 {
-    if (!FC_SPEC_DYNAMIC || sp.diag) return false;
+    if (sp.diag) return false;
     // Two surface types keep the static schedule unless the caller asks (option dyn_min_tiles): a t tile is 128 KB of traffic
     // and ~9 us of a team's time there, claims are coarse against 132 tiles per CTA, and consecutive static steps hand over
     // per CTA -- measured on C5 (10^7 cells, call 14, two repetitions): static 0.908 / 0.909 ms, dynamic 0.922 / 0.926 ms.
     if (sp.ns > 1 && sp.dyn <= 0) return false;
-    const int64_t min_tiles = sp.dyn > 0 ? sp.dyn : FC_SPEC_DYN_MIN_TILES;      // (before the launch sp.dyn carries the caller's threshold)
+    const int64_t min_tiles = sp.dyn > 0 ? sp.dyn : kSpecDynMinTiles;      // (before the launch sp.dyn carries the caller's threshold)
     return (int64_t)sp.ntiles[0] + sp.ntiles[1] + sp.ntiles[2] >= min_tiles * spec_grid(sp);
 }
 
@@ -1629,8 +1543,7 @@ static cudaError_t spec_launch_t(const SpecPlan &sp, int grid, cudaStream_t stre
     cfg.stream = stream;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    static const int no_pdl = getenv("FC_NO_PDL") ? atoi(getenv("FC_NO_PDL")) : 0;      // tuning aid
-    attr[0].val.programmaticStreamSerializationAllowed = no_pdl ? 0 : 1;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, flux_spec_kernel<SET, NS, DIAG, DYN>, sp);
@@ -1641,7 +1554,7 @@ static cudaError_t spec_launch_d(const SpecPlan &sp, int grid, cudaStream_t stre
 {
     if (sp.diag >= 2) return spec_launch_t<SET, NS, 2, false>(sp, grid, stream);
     if (sp.diag == 1) return spec_launch_t<SET, NS, 1, false>(sp, grid, stream);
-    if (FC_SPEC_DYNAMIC && sp.dyn) return spec_launch_t<SET, NS, 0, true>(sp, grid, stream);
+    if (sp.dyn) return spec_launch_t<SET, NS, 0, true>(sp, grid, stream);
     return spec_launch_t<SET, NS, 0, false>(sp, grid, stream);
 }
 

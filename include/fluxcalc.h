@@ -264,8 +264,7 @@ int fc_step_all(fc_context *ctx, int64_t current_step_time);
  * only) -- the time loop of flux_calculator.F90:859-1028 for a host that keeps its fields on the device.  The steps of one
  * calendar month differ in nothing (the month selects the bias slab, calculate.F90:66-73): they are issued as replays of
  * one CUDA graph of 32 step launches per month, the remainder directly.  Results are bit-identical to nsteps calls of
- * fc_step_all.  With diagnostics only the LAST step's values can be read afterwards.  Option "graphs" = 0 issues
- * every step directly. */
+ * fc_step_all.  With diagnostics only the LAST step's values can be read afterwards. */
 int fc_run_steps(fc_context *ctx, int64_t t0, int64_t timestep, int nsteps);
 
 int fc_synchronize(fc_context *ctx);
@@ -283,15 +282,13 @@ int fc_kernel_time_ms(fc_context *ctx, double *total_ms, int64_t *count);
 /* options: "early_loads" (0/1, default 1: a step that directly follows another step of this context on its stream may
  *          fill its shared-memory ring before the previous step has finished -- steps write no input array; set
  *          "stream_touched" = 1 after enqueuing own work that writes bound arrays on fc_get_stream()),
- *          "graphs" (0/1, default 1: fc_run_steps replays CUDA graphs), "dyn_min_tiles" (tiles per CTA from which the
- *          specialised kernel without diagnostics claims tiles dynamically; 0 = default: 48 with one surface type, never
- *          with two),
+ *          "dyn_min_tiles" (tiles per CTA from which the specialised kernel without diagnostics claims tiles dynamically;
+ *          0 = default: 48 with one surface type, never with two),
  *          "force_generic" (0/1: use the op-list interpreter kernels instead of the fused kernel),
  *          "pin_host" (0/1: cudaHostRegister bound host arrays), "h2d_chunks" (pipeline depth of the
  *          host-pointer path), "diagnostics" (0 off, 1 area-weighted sums, 2 sums + min/max),
  *          "profile_kernel" (0 off, n: time every n-th fused launch), "staged" (specialised persistent kernel: 0 never,
- *          >= 1 (default) whenever the plan fits),
- *          "prefetch_distance" (L2 prefetch look-ahead of the direct kernel in 512-cell blocks, default 0) */
+ *          >= 1 (default) whenever the plan fits) */
 int fc_set_option(fc_context *ctx, const char *name, int64_t value);
 int64_t fc_get_info(const fc_context *ctx, const char *name);
 /* info names: "launches" (kernel launches issued so far), "fused" (1 if the fused kernel serves
