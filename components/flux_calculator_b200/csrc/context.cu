@@ -1013,6 +1013,39 @@ static int run_ops(fc_context *c, const std::vector<HOp> &ops)
 // fused plan builder
 // ---------------------------------------------------------------------------------------------
 
+// chunks of the host-pointer pipeline.  Its depth: the first chunk's upload and the last chunk's download are exposed, so even
+// a small shard (the 8-GPU share of a 10^7-cell grid is 1.25 * 10^6 cells) gets at least 8 chunks; tiny grids are not worth
+// splitting
+static int pipeline_chunks(const fc_context *c)
+{
+    const int64_t nmax = std::max(c->n[1], std::max(c->n[2], c->n[3]));
+    return c->h2d_chunks > 0 ? std::min(c->h2d_chunks, kMaxChunks)
+                             : (nmax < 65536 ? 1 : (int)std::min<int64_t>(kMaxChunks, std::max<int64_t>(8, nmax / 262144)));
+}
+
+// chunk boundaries of the host-pointer pipeline: 256-byte aligned starts, the last chunk takes the remainder
+static void chunk_range(const fc_context *c, int k, int K, int64_t c0[4], int64_t c1[4])
+{
+    for (int g = 1; g <= 3; ++g) {
+        c0[g] = (K == 1) ? 0 : ((c->n[g] * k / K) & ~int64_t(31));
+        c1[g] = (k == K - 1) ? c->n[g] : ((c->n[g] * (k + 1) / K) & ~int64_t(31));
+    }
+}
+
+// how the plan launches as one device-resident step and as the chunks of the host-pointer pipeline
+static void resolve_bundle(const fc_context *c, FusedBundle &F)
+{
+    const int64_t zero[3] = {0, 0, 0}, n[3] = {c->n[1], c->n[2], c->n[3]};
+    F.step = resolve_fused(F.plan, zero, n, c->use_staged, c->dyn_min_tiles);
+    const int K = pipeline_chunks(c);
+    for (int k = 0; k < K; ++k) {
+        int64_t c0[4], c1[4];
+        chunk_range(c, k, K, c0, c1);
+        const int64_t first[3] = {c0[1], c0[2], c0[3]}, cells[3] = {c1[1] - c0[1], c1[2] - c0[2], c1[3] - c0[3]};
+        F.chunks.push_back(resolve_fused(F.plan, first, cells, c->use_staged, c->dyn_min_tiles));
+    }
+}
+
 static bool build_fused(fc_context *c, bool do_early, bool do_normal, FusedBundle &F)
 {
     F = FusedBundle();
@@ -1022,10 +1055,6 @@ static bool build_fused(fc_context *c, bool do_early, bool do_normal, FusedBundl
     P.do_early = do_early;
     P.do_normal = do_normal;
     P.c = c->consts;
-    for (int g = 0; g < 3; ++g) {
-        P.cell0[g] = 0;
-        P.cells[g] = c->n[g + 1];
-    }
     P.t.n = c->n[1];
     P.uv[0].n = c->n[2];
     P.uv[1].n = c->n[3];
@@ -1254,10 +1283,9 @@ static bool build_fused(fc_context *c, bool do_early, bool do_normal, FusedBundl
         P.diag_n = (int)F.diag_slots.size();
         if (P.diag_n == 0) P.diag = 0;
     }
-    P.staged = c->use_staged;
-    P.dyn_min_tiles = c->dyn_min_tiles;
     F.in_bufs.assign(ins.begin(), ins.end());
     F.out_bufs.assign(outs.begin(), outs.end());
+    resolve_bundle(c, F);
     F.ok = true;
     return true;
 }
@@ -1384,36 +1412,13 @@ extern "C" int fc_average_across_surface_types(fc_context *c, int g, int idx)
 // ---------------------------------------------------------------------------------------------
 // fused steps
 // ---------------------------------------------------------------------------------------------
-// chunk boundaries of the host-pointer pipeline: 256-byte aligned starts, the last chunk takes the remainder
-static void chunk_range(const fc_context *c, int k, int K, int64_t c0[4], int64_t c1[4])
-{
-    for (int g = 1; g <= 3; ++g) {
-        c0[g] = (K == 1) ? 0 : ((c->n[g] * k / K) & ~int64_t(31));
-        c1[g] = (k == K - 1) ? c->n[g] : ((c->n[g] * (k + 1) / K) & ~int64_t(31));
-    }
-}
-
-static FusedPlan chunk_plan(const fc_context *c, const FusedPlan &P, int k, int K)
-{
-    FusedPlan Q = P;
-    if (K > 1) {
-        int64_t c0[4], c1[4];
-        chunk_range(c, k, K, c0, c1);
-        for (int g = 0; g < 3; ++g) {
-            Q.cell0[g] = c0[g + 1];
-            Q.cells[g] = c1[g + 1] - c0[g + 1];
-        }
-    }
-    return Q;
-}
-
 // Diagnostics storage for a step issued as K launches (K = 1: device-resident; K > 1: chunks of the host-pointer
 // pipeline, which run concurrently on three streams): every chunk owns its partial rows, its reduce scratch, its
-// last-CTA counter and its result vector; diag_combine folds the K vectors in chunk order into P.diag_out.
-static int ensure_diag_storage(fc_context *c, FusedPlan &P, int K)
+// last-CTA counter and its result vector; diag_combine folds the K vectors in chunk order into a.diag_out.
+static int ensure_diag_storage(fc_context *c, const FusedPlan &P, const FusedLaunch *L, int K, FusedStepArgs &a)
 {
     int64_t rows = 1;
-    for (int k = 0; k < K; ++k) rows = std::max(rows, fused_diag_rows(chunk_plan(c, P, k, K)));
+    for (int k = 0; k < K; ++k) rows = std::max(rows, L[k].diag_rows);
     const int planes = P.diag >= 2 ? 3 : 1;
     const size_t stride = (size_t)planes * P.diag_n * (size_t)rows + (size_t)diag_tmp_doubles(rows, P.diag_n);
     // K = 1: two sets, alternating by step -- the rows of step k are folded while step k + 1 writes its own (DiagFold)
@@ -1438,8 +1443,8 @@ static int ensure_diag_storage(fc_context *c, FusedPlan &P, int K)
         CUDA_TRY(c, cudaMalloc(&c->diag_chunk_out, sizeof(double) * kDiagSlots * 3 * kMaxChunks));
         CUDA_TRY(c, cudaMemsetAsync(c->diag_chunk_out, 0, sizeof(double) * kDiagSlots * 3 * kMaxChunks, c->stream));
     }
-    P.diag_partials = c->diag_partials;
-    P.diag_rows = rows;
+    a.diag_partials = c->diag_partials;
+    a.diag_rows = rows;
     if (K == 1) c->diag_rows_1 = rows;
     // result buffer of this step; if its previous all-reduce is still in flight on the side stream, wait for it
     const int b = c->diag_cur ^ 1;
@@ -1447,46 +1452,45 @@ static int ensure_diag_storage(fc_context *c, FusedPlan &P, int K)
         CUDA_TRY(c, cudaStreamWaitEvent(c->stream, c->ev_comm[b], 0));
         c->comm_busy[b] = false;
     }
-    P.diag_out = c->diag_buf[b];
+    a.diag_out = c->diag_buf[b];
     return FC_OK;
 }
 
 // chunk k's view of the diagnostics storage
-static void diag_chunk_view(const fc_context *c, const FusedPlan &P, int k, int K, FusedPlan &Q)
+static void diag_chunk_view(const fc_context *c, const FusedStepArgs &a, int k, int K, FusedStepArgs &q)
 {
-    Q.diag_partials = c->diag_partials + (size_t)k * c->diag_chunk_stride;
-    Q.diag_rows = P.diag_rows;
-    Q.diag_out = (K == 1) ? P.diag_out : c->diag_chunk_out + (size_t)k * 3 * kDiagSlots;
+    q.diag_partials = c->diag_partials + (size_t)k * c->diag_chunk_stride;
+    q.diag_rows = a.diag_rows;
+    q.diag_out = (K == 1) ? a.diag_out : c->diag_chunk_out + (size_t)k * 3 * kDiagSlots;
 }
 
-static double *diag_tmp(const FusedPlan &Q)
+static double *diag_tmp(const FusedPlan &P, const FusedStepArgs &a)
 {
-    const int planes = Q.diag >= 2 ? 3 : 1;
-    return Q.diag_partials + (size_t)planes * Q.diag_n * (size_t)Q.diag_rows;
+    const int planes = P.diag >= 2 ? 3 : 1;
+    return a.diag_partials + (size_t)planes * P.diag_n * (size_t)a.diag_rows;
 }
 
-// partial rows of launch Q -> Q.diag_out, on the stream Q was launched on; a no-op launch-wise when the specialised
-// kernel already reduced them itself
-static int finalize_chunk(fc_context *c, const FusedPlan &Q, cudaStream_t s)
+// partial rows of a generic launch -> a.diag_out, on the stream it was launched on
+static int finalize_chunk(fc_context *c, const FusedPlan &P, const FusedLaunch &L, const FusedStepArgs &a, cudaStream_t s)
 {
     int nl = 0;
-    if (launch_diag_finalize(Q, diag_tmp(Q), Q.diag_out, s, &nl)) return fail(c, FC_ERR_CUDA, "diag finalize launch failed");
+    if (launch_diag_finalize(P, L, a, diag_tmp(P, a), s, &nl)) return fail(c, FC_ERR_CUDA, "diag finalize launch failed");
     c->launches += nl;
     return FC_OK;
 }
 
-// the rows a specialised launch of Q leaves behind, as a fold request
-static DiagFold make_fold(const FusedPlan &Q)
+// the rows a specialised launch leaves behind, as a fold request
+static DiagFold make_fold(const FusedPlan &P, const FusedLaunch &L, const FusedStepArgs &a)
 {
     DiagFold f;
     memset(&f, 0, sizeof f);
-    f.rows = Q.diag_partials;
-    f.row_stride = Q.diag_rows;
-    f.plane = (int64_t)Q.diag_n * Q.diag_rows;
-    f.nrows = (int)fused_diag_rows(Q);
-    f.nslots = Q.diag_n;
-    f.level = Q.diag;
-    f.out = Q.diag_out;
+    f.rows = a.diag_partials;
+    f.row_stride = a.diag_rows;
+    f.plane = (int64_t)P.diag_n * a.diag_rows;
+    f.nrows = (int)L.diag_rows;
+    f.nslots = P.diag_n;
+    f.level = P.diag;
+    f.out = a.diag_out;
     return f;
 }
 
@@ -1504,17 +1508,16 @@ int flush_fold(fc_context *c)
 }
 }  // namespace fc
 
-// bookkeeping once the step's result vector (P.diag_out = diag_buf[next]) is issued
-static void diag_step_done(fc_context *c, const FusedPlan &P, const FusedBundle &F)
+// bookkeeping once the step's result vector (diag_buf[next]) is issued
+static void diag_step_done(fc_context *c, const FusedBundle &F)
 {
     c->diag_cur ^= 1;
     c->diag_active = F.diag_slots;
     c->diag_valid = false;
     c->diag_global = false;
-    c->diag_level = P.diag;
+    c->diag_level = F.plan.diag;
 }
 
-// dynamic schedule: give launch Q claim counter `slot`; returns by how much the launch will advance it
 static int ensure_tile_counters(fc_context *c)
 {
     if (!c->tile_ctr) {
@@ -1525,37 +1528,30 @@ static int ensure_tile_counters(fc_context *c)
     return FC_OK;
 }
 
-static int attach_tile_counter(fc_context *c, FusedPlan &Q, int slot, unsigned int *claims)
+// dynamic schedule: give launch L claim counter `slot` (the caller advances the counter's base by L.claims)
+static int attach_tile_counter(fc_context *c, const FusedLaunch &L, FusedStepArgs &a, int slot)
 {
-    *claims = fused_dyn_claims(Q);
-    if (*claims == 0) return FC_OK;
+    if (L.claims == 0) return FC_OK;
     if (int rc = ensure_tile_counters(c)) return rc;
-    Q.tile_counter = c->tile_ctr + slot;
-    Q.tile_base = c->tile_base[slot];
+    a.tile_counter = c->tile_ctr + slot;
+    a.tile_base = c->tile_base[slot];
     return FC_OK;
 }
 
-// geometry facts of a bundle's plan that do not change from step to step (cached: each costs a plan build)
-static void bundle_geometry(FusedBundle &F, const FusedPlan &P)
-{
-    const int key = 1 + (int)(reinterpret_cast<uintptr_t>(P.t.bias) & 15u);      // (the bias slab is the only pointer that moves between steps)
-    if (F.geom_cached == key) return;
-    F.spec = fused_uses_spec(P) != 0;
-    F.claims = F.spec ? fused_dyn_claims(P) : 0u;
-    F.fills = F.spec && fused_fills_device(P) != 0;
-    F.geom_cached = key;
-}
-
-// one device-resident step on the context's stream.  gstep < 0: an ordinary step.  gstep >= 0: step number gstep of a
-// sequence that is being captured into a CUDA graph (fc_run_steps): nothing here may depend on state that changes
-// between two launches of that graph -- no fold of the previous step's rows (only the last step's diagnostics are
-// ever read; the caller registers them after the graph), one row set, tile counters that the graph's leading memset
-// node zeroes (step s uses counter s mod 2 at base (s / 2) * claims), no event records, no allocation.
-static int launch_resident(fc_context *c, FusedBundle &F, FusedPlan &P, int gstep)
+// one device-resident step on the context's stream.  Which kernel runs and how it is scheduled was decided when the plan
+// was prepared (F.step, kernels.cu: resolve_fused); what is left here is this step's arguments.  gstep < 0: an ordinary
+// step.  gstep >= 0: step number gstep of a sequence that is being captured into a CUDA graph (fc_run_steps): nothing here
+// may depend on state that changes between two launches of that graph -- no fold of the previous step's rows (only the
+// last step's diagnostics are ever read; the caller registers them after the graph), one row set, tile counters that the
+// graph's leading memset node zeroes (step s uses counter s mod 2 at base (s / 2) * claims), no event records, no allocation.
+static int launch_resident(fc_context *c, const FusedBundle &F, const double *bias, int gstep)
 {
     const bool graph = gstep >= 0;
-    bundle_geometry(F, P);
-    const bool spec = F.spec;
+    const FusedPlan &P = F.plan;
+    const FusedLaunch &L = F.step;
+    const bool spec = L.spec;
+    FusedStepArgs a{};
+    a.bias = bias;
     int nlaunch = 0;
     // rows of the previous specialised step that nobody folded yet: this launch folds them while its ring fills,
     // unless it is not that kind of launch
@@ -1563,30 +1559,28 @@ static int launch_resident(fc_context *c, FusedBundle &F, FusedPlan &P, int gste
         if (int rc = flush_fold(c)) return rc;
     if (P.diag) {
         if (!graph)
-            if (int rc = ensure_diag_storage(c, P, 1)) return rc;
+            if (int rc = ensure_diag_storage(c, P, &L, 1, a)) return rc;
         const int b = c->diag_cur ^ 1;
-        P.diag_partials = c->diag_partials;
-        P.diag_rows = c->diag_rows_1;
-        P.diag_out = c->diag_buf[b];
-        diag_chunk_view(c, P, graph ? 0 : (c->row_set ^= 1), 1, P);
-        if (!graph && c->fold_pending) P.fold_prev = c->fold;
+        a.diag_partials = c->diag_partials;
+        a.diag_rows = c->diag_rows_1;
+        a.diag_out = c->diag_buf[b];
+        diag_chunk_view(c, a, graph ? 0 : (c->row_set ^= 1), 1, a);
+        if (!graph && c->fold_pending) a.fold_prev = c->fold;
     }
-    P.early_loads = (spec && c->early_loads && (graph ? gstep > 0 : c->tail_own_step)) ? 1 : 0;
+    a.early_loads = (spec && c->early_loads && (graph ? gstep > 0 : c->tail_own_step)) ? 1 : 0;
     // dynamic schedule: consecutive steps alternate between two counters, because the producers of a step may claim
     // while the previous step still runs.  That holds for at most two steps at a time only if this step's grid
     // fills the device (a third step finds no room before the first has left); smaller grids wait first.
-    const unsigned int claims = F.claims;
+    const unsigned int claims = L.claims;
     const int tslot = kMaxChunks + (graph ? (gstep & 1) : (c->tile_par ^= 1));
     if (claims && !graph)
         if (int rc = ensure_tile_counters(c)) return rc;
     if (claims) {
-        P.tile_counter = c->tile_ctr + tslot;
-        P.tile_base = graph ? (unsigned int)(gstep >> 1) * claims : c->tile_base[tslot];
+        a.tile_counter = c->tile_ctr + tslot;
+        a.tile_base = graph ? (unsigned int)(gstep >> 1) * claims : c->tile_base[tslot];
     }
-    if (claims && !F.fills) P.early_loads = 0;
+    if (claims && !L.fills) a.early_loads = 0;
     // static schedule: record per-CTA completion, and hand over per CTA if the previous launch of the stream was this plan
-    P.chain = 0;
-    P.chain_done = nullptr;
     if (spec && !claims && !graph) {
         if (!c->chain_done) {
             const size_t nb = sizeof(unsigned int) * (size_t)std::max(spec_capacity(1), spec_capacity(2));
@@ -1594,10 +1588,10 @@ static int launch_resident(fc_context *c, FusedBundle &F, FusedPlan &P, int gste
             CUDA_TRY(c, cudaMemsetAsync(c->chain_done, 0, nb, c->stream));
             c->tail_own_step = false;
         }
-        P.chain_done = c->chain_done;
-        P.chain_seq = ++c->chain_seq;
-        P.chain = (c->chain_steps && c->early_loads && c->tail_own_step && c->chain_key == (const void *)&F && F.fills) ? 1 : 0;
-        if (!P.chain && !c->tail_own_step) P.early_loads = 0;
+        a.chain_done = c->chain_done;
+        a.chain_seq = ++c->chain_seq;
+        a.chain = (c->chain_steps && c->early_loads && c->tail_own_step && c->chain_key == (const void *)&F && L.fills) ? 1 : 0;
+        if (!a.chain && !c->tail_own_step) a.early_loads = 0;
     }
     cudaEvent_t e0 = nullptr, e1 = nullptr;
     if (!graph && c->profile_kernel && c->prof_used < 8192 && (c->prof_seq++ % c->profile_kernel) == 0) {
@@ -1611,7 +1605,7 @@ static int launch_resident(fc_context *c, FusedBundle &F, FusedPlan &P, int gste
         c->prof_used += 2;
         CUDA_TRY(c, cudaEventRecord(e0, c->stream));
     }
-    if (launch_fused(P, c->stream, &nlaunch)) return fail(c, FC_ERR_CUDA, "fused launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+    if (launch_fused(P, L, a, c->stream, &nlaunch)) return fail(c, FC_ERR_CUDA, "fused launch failed: %s", cudaGetErrorString(cudaGetLastError()));
     if (e1) CUDA_TRY(c, cudaEventRecord(e1, c->stream));
     c->launches += nlaunch;
     if (!graph) {
@@ -1623,13 +1617,13 @@ static int launch_resident(fc_context *c, FusedBundle &F, FusedPlan &P, int gste
     if (P.diag) {
         if (spec) {
             if (!graph) {
-                c->fold = make_fold(P);
+                c->fold = make_fold(P, L, a);
                 c->fold_pending = true;
             }
-        } else if (int rc = finalize_chunk(c, P, c->stream)) {
+        } else if (int rc = finalize_chunk(c, P, L, a, c->stream)) {
             return rc;
         }
-        if (!graph) diag_step_done(c, P, F);
+        if (!graph) diag_step_done(c, F);
     }
     if (!F.extra.empty())
         if (int rc = run_ops(c, F.extra)) return rc;
@@ -1638,10 +1632,8 @@ static int launch_resident(fc_context *c, FusedBundle &F, FusedPlan &P, int gste
 
 static int run_fused(fc_context *c, FusedBundle &F, bool async_device_only)
 {
-    FusedPlan P = F.plan;
-    if (P.t.bias) {
-        P.t.bias = bias_slab(c);
-    }
+    const FusedPlan &P = F.plan;
+    const double *bias = P.t.bias ? bias_slab(c) : nullptr;
     bool any_host = false;
     for (int b : F.in_bufs) any_host = any_host || !c->bufs[b].user_is_device;
     for (int b : F.out_bufs) any_host = any_host || !c->bufs[b].user_is_device;
@@ -1651,15 +1643,11 @@ static int run_fused(fc_context *c, FusedBundle &F, bool async_device_only)
     if (async_device_only && any_host) return fail(c, FC_ERR_STATE, "fc_run_steps needs device-resident fields (bind device pointers)");
     int nlaunch = 0;
 
-    if (!any_host) return launch_resident(c, F, P, -1);
+    if (!any_host) return launch_resident(c, F, bias, -1);
 
     // host-pointer mode: chunked H2D -> kernel -> D2H pipeline over three streams (copy engines
     // and SMs overlap; inputs of chunk k+1 travel while chunk k computes and chunk k-1 returns)
-    int64_t nmax = std::max(c->n[1], std::max(c->n[2], c->n[3]));
-    // pipeline depth: the first chunk's upload and the last chunk's download are exposed, so even a small shard (the 8-GPU
-    // share of a 10^7-cell grid is 1.25 * 10^6 cells) gets at least 8 chunks; tiny grids are not worth splitting
-    const int K = c->h2d_chunks > 0 ? std::min(c->h2d_chunks, kMaxChunks)
-                  : (nmax < 65536 ? 1 : (int)std::min<int64_t>(kMaxChunks, std::max<int64_t>(8, nmax / 262144)));
+    const int K = (int)F.chunks.size();
     // what travels: inputs the host may have rewritten (everything not marked static, and static arrays not uploaded
     // yet), results the host will read (everything computed, or with option "download" = 1 only the registered output
     // fields -- what the reference hands to oasis_put, flux_calculator.F90:909-936,999-1026)
@@ -1677,9 +1665,11 @@ static int run_fused(fc_context *c, FusedBundle &F, bool async_device_only)
         for (int b : F.out_bufs)
             if (!c->bufs[b].user_is_device && (!sent_only || sent.count(b))) down.push_back(b);
     }
+    FusedStepArgs a{};
+    a.bias = bias;
     if (int rc = flush_fold(c)) return rc;
     if (P.diag)
-        if (int rc = ensure_diag_storage(c, P, K)) return rc;
+        if (int rc = ensure_diag_storage(c, P, F.chunks.data(), K, a)) return rc;
     c->tail_own_step = false;
     CUDA_TRY(c, cudaStreamSynchronize(c->stream));
     for (int k = 0; k < K; ++k) {
@@ -1693,17 +1683,17 @@ static int run_fused(fc_context *c, FusedBundle &F, bool async_device_only)
             CUDA_TRY(c, cudaMemcpyAsync(B.dev + c0[B.grid], B.user + c0[B.grid], (size_t)cnt * sizeof(double), cudaMemcpyHostToDevice, s));
             c->h2d_bytes += cnt * (int64_t)sizeof(double);
         }
-        FusedPlan Q = chunk_plan(c, P, k, K);
-        if (P.diag) diag_chunk_view(c, P, k, K, Q);
-        unsigned int claims = 0;
-        if (int rc = attach_tile_counter(c, Q, k, &claims)) return rc;
-        c->tile_base[k] += claims;
-        if (launch_fused(Q, s, &nlaunch)) return fail(c, FC_ERR_CUDA, "fused launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+        const FusedLaunch &L = F.chunks[(size_t)k];
+        FusedStepArgs q = a;
+        if (P.diag) diag_chunk_view(c, a, k, K, q);
+        if (int rc = attach_tile_counter(c, L, q, k)) return rc;
+        c->tile_base[k] += L.claims;
+        if (launch_fused(P, L, q, s, &nlaunch)) return fail(c, FC_ERR_CUDA, "fused launch failed: %s", cudaGetErrorString(cudaGetLastError()));
         if (P.diag) {
-            if (fused_uses_spec(Q)) {      // the chunk's rows -> the chunk's result vector, right behind it on its stream
-                if (launch_diag_fold(make_fold(Q), s)) return fail(c, FC_ERR_CUDA, "diag fold launch failed");
+            if (L.spec) {      // the chunk's rows -> the chunk's result vector, right behind it on its stream
+                if (launch_diag_fold(make_fold(P, L, q), s)) return fail(c, FC_ERR_CUDA, "diag fold launch failed");
                 nlaunch += 1;
-            } else if (int rc = finalize_chunk(c, Q, s)) {
+            } else if (int rc = finalize_chunk(c, P, L, q, s)) {
                 return rc;
             }
         }
@@ -1720,10 +1710,10 @@ static int run_fused(fc_context *c, FusedBundle &F, bool async_device_only)
     for (int b : up) c->bufs[b].dev_valid = true;
     if (P.diag) {
         if (K > 1) {      // fold the chunks' result vectors in chunk order
-            if (launch_diag_combine(c->diag_chunk_out, K, P.diag_out, c->stream)) return fail(c, FC_ERR_CUDA, "diag combine launch failed");
+            if (launch_diag_combine(c->diag_chunk_out, K, a.diag_out, c->stream)) return fail(c, FC_ERR_CUDA, "diag combine launch failed");
             c->launches += 1;
         }
-        diag_step_done(c, P, F);
+        diag_step_done(c, F);
     }
     if (!F.extra.empty())
         if (int rc = run_ops(c, F.extra)) return rc;
@@ -1825,26 +1815,23 @@ extern "C" int fc_step_all(fc_context *c, int64_t t) { return step_impl(c, 2, t,
 namespace {
 constexpr int kGraphSteps = 32;      // step launches per graph (even: the tile counters alternate)
 
-int capture_steps(fc_context *c, FusedBundle &F, int month, int nsteps, cudaGraphExec_t *exec)
+int capture_steps(fc_context *c, const FusedBundle &F, int month, int nsteps, cudaGraphExec_t *exec)
 {
-    FusedPlan P0 = F.plan;
-    if (P0.t.bias) P0.t.bias = c->corr_dev + (size_t)(month - 1) * (size_t)corr_stride(c->n[1]);
+    const double *bias = F.plan.t.bias ? c->corr_dev + (size_t)(month - 1) * (size_t)corr_stride(c->n[1]) : nullptr;
     // everything that allocates or synchronises happens before the capture
     if (int rc = flush_fold(c)) return rc;
-    bundle_geometry(F, P0);
-    if (F.claims)
+    if (F.step.claims)
         if (int rc = ensure_tile_counters(c)) return rc;
-    if (P0.diag)
-        if (int rc = ensure_diag_storage(c, P0, 1)) return rc;
+    if (F.plan.diag) {
+        FusedStepArgs unused{};
+        if (int rc = ensure_diag_storage(c, F.plan, &F.step, 1, unused)) return rc;
+    }
     cudaGraph_t graph = nullptr;
     CUDA_TRY(c, cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal));
     int rc = FC_OK;
-    if (F.claims && cudaMemsetAsync(c->tile_ctr + kMaxChunks, 0, 2 * sizeof(unsigned int), c->stream) != cudaSuccess)
+    if (F.step.claims && cudaMemsetAsync(c->tile_ctr + kMaxChunks, 0, 2 * sizeof(unsigned int), c->stream) != cudaSuccess)
         rc = fail(c, FC_ERR_CUDA, "fc_run_steps: memset node failed");
-    for (int s = 0; s < nsteps && rc == FC_OK; ++s) {
-        FusedPlan P = P0;
-        rc = launch_resident(c, F, P, s);
-    }
+    for (int s = 0; s < nsteps && rc == FC_OK; ++s) rc = launch_resident(c, F, bias, s);
     const cudaError_t e = cudaStreamEndCapture(c->stream, &graph);
     if (rc != FC_OK) {
         if (graph) cudaGraphDestroy(graph);
@@ -1891,21 +1878,20 @@ extern "C" int fc_run_steps(fc_context *c, int64_t t0, int64_t dt, int nsteps)
             run -= kGraphSteps;
             // state as the graph leaves it: time, tile counters, the last step's diagnostics rows (set 0) not folded yet
             c->time = t0 + (int64_t)(k - 1) * dt;
-            if (F.claims) c->tile_base[kMaxChunks] = c->tile_base[kMaxChunks + 1] = (unsigned int)(kGraphSteps / 2) * F.claims;
-            c->tail_own_step = F.spec && F.extra.empty();
+            if (F.step.claims) c->tile_base[kMaxChunks] = c->tile_base[kMaxChunks + 1] = (unsigned int)(kGraphSteps / 2) * F.step.claims;
+            c->tail_own_step = F.step.spec && F.extra.empty();
             c->chain_key = nullptr;
             if (F.plan.diag) {
-                FusedPlan P = F.plan;
-                P.diag_partials = c->diag_partials;
-                P.diag_rows = c->diag_rows_1;
-                P.diag_out = c->diag_buf[c->diag_cur ^ 1];
-                diag_chunk_view(c, P, 0, 1, P);
+                FusedStepArgs a{};
+                a.diag_partials = c->diag_partials;
+                a.diag_rows = c->diag_rows_1;
+                a.diag_out = c->diag_buf[c->diag_cur ^ 1];
                 c->row_set = 0;
-                if (F.spec) {
-                    c->fold = make_fold(P);
+                if (F.step.spec) {
+                    c->fold = make_fold(F.plan, F.step, a);
                     c->fold_pending = true;
                 }
-                diag_step_done(c, P, F);
+                diag_step_done(c, F);
             }
         }
         for (int r = 0; r < run; ++r, ++k)
@@ -1969,9 +1955,7 @@ extern "C" int64_t fc_get_info(const fc_context *c, const char *name)
     }
     if (!strcmp(name, "fused")) return (!c->dirty && c->fused[2].ok) ? 1 : 0;
     if (!strcmp(name, "spec_kernel")) {   // fc_step_all runs on the specialised persistent kernel (spec_kernel.cu)
-        if (c->dirty || !c->fused[2].ok) return 0;
-        cudaSetDevice(c->device);
-        return fused_uses_spec(c->fused[2].plan);
+        return (!c->dirty && c->fused[2].ok && c->fused[2].step.spec) ? 1 : 0;
     }
     if (!strcmp(name, "fused_early")) return (!c->dirty && c->fused[0].ok) ? 1 : 0;
     if (!strcmp(name, "fused_normal")) return (!c->dirty && c->fused[1].ok) ? 1 : 0;

@@ -57,10 +57,9 @@ enum Quantity { Q_QSUR_T = 0, Q_QSUR_U, Q_QSUR_V, Q_MEVA, Q_HLAT, Q_HSEN, Q_MOM,
 
 struct FusedBundle {
     bool ok = false;
-    int geom_cached = 0;      // 0: not yet; else 1 + alignment of the bias slab the facts below were computed for
-    bool spec = false, fills = false;   // step-invariant facts of the plan's geometry (context.cu: bundle_geometry)
-    unsigned int claims = 0;
     FusedPlan plan;
+    FusedLaunch step;                     // how the plan launches as a device-resident step (kernels.cu: resolve_fused)
+    std::vector<FusedLaunch> chunks;      // ... and as the chunks of the host-pointer pipeline
     std::vector<int> in_bufs, out_bufs;   // buffers to upload / download in host-pointer mode
     std::vector<HOp> extra;               // averaging of pass-through variables (run after the fused launch)
     // diagnostics slot -> (surface type, grid, var) of the active slots, compact order
@@ -154,7 +153,6 @@ struct fc_context {
     bool strict = false;
     fc::Consts consts;
     fc::FusedBundle fused[3];    // 0 early, 1 normal, 2 all
-    int fused_month = 0;         // month the bias pointer in the fused plans refers to
 
     // diagnostics storage
     double *diag_partials = nullptr;

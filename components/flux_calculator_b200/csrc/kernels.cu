@@ -415,17 +415,6 @@ __device__ __forceinline__ bool uv_chain(const FusedPlan &p, const FusedUV &g, i
     return bad;
 }
 
-// FULL = true : every thread owns V whole cells and every array is 16-byte aligned (128-bit accesses only);
-//               launched over floor(cells/V) cell vectors per grid.
-// FULL = false: guarded scalar accesses; launched over the ragged remainder (cells % V) of each grid, or over
-//               everything when a bound array is not 16-byte aligned.  first[] = first cell of this launch.
-struct LaunchGeom {
-    int nb_t, nb_u;          // blocks of the t / u grid (the rest is the v grid)
-    int64_t first[3];        // first cell handled by this launch on each grid
-    int64_t count[3];        // cells handled by this launch on each grid
-    int64_t row0;            // first diagnostics row of this launch
-};
-
 // cold, out of line: every lane of the warp that called recomputes its V cells with the IEEE policy (identical bits for the
 // lanes whose operands were in range: ExactVec's exp / pow fall back to the lock-step sequences there) and, with
 // diagnostics, the warp's row is rebuilt by the same trees.  Scalars only: nothing of the hot path's state is passed.
@@ -664,12 +653,12 @@ __global__ void regrid_csr_kernel(const int64_t *__restrict__ row_ptr, const int
 // ---------------------------------------------------------------------------------------------
 // launchers
 // ---------------------------------------------------------------------------------------------
-static bool plan_aligned(const FusedPlan &p)
+static bool plan_aligned(const FusedPlan &p, const int64_t first[3])
 {
     auto ok = [](const void *q, int64_t cell0) { return q == nullptr || ((reinterpret_cast<uintptr_t>(q) + cell0 * 8) & 15) == 0; };
     bool a = true;
     const FusedT &t = p.t;
-    const int64_t c0 = p.cell0[0];
+    const int64_t c0 = first[0];
     a = a && ok(t.rsdd, c0) && ok(t.bias, c0) && ok(t.area, c0) && ok(t.avg_qsur, c0) && ok(t.avg_meva, c0) &&
         ok(t.avg_hlat, c0) && ok(t.avg_hsen, c0) && ok(t.avg_rbbr, c0) && ok(t.avg_rsdr, c0);
     for (int i = 0; i < p.S; ++i) {
@@ -680,7 +669,7 @@ static bool plan_aligned(const FusedPlan &p)
     }
     for (int g = 0; g < 2; ++g) {
         const FusedUV &u = p.uv[g];
-        const int64_t cg = p.cell0[g + 1];
+        const int64_t cg = first[g + 1];
         a = a && ok(u.area, cg) && ok(u.avg_qsur, cg) && ok(u.avg_mom, cg);
         for (int i = 0; i < p.S; ++i) {
             const FusedUVType &y = u.ty[i];
@@ -691,138 +680,116 @@ static bool plan_aligned(const FusedPlan &p)
     return a;
 }
 
-// geometry of the (up to) two launches of one fused step: whole 512-cell blocks through the 128-bit kernel
-// (specialised persistent kernel or generic direct-load kernel), the ragged remainder (or everything, if an array is
-// misaligned) through the guarded kernel
-struct FusedGeom {
-    LaunchGeom main, tail;
-    int nb_main, nb_tail;
-    bool spec;           // main part runs on the specialised persistent kernel (spec_kernel.cu)
-    bool diag_accum;     // ... which accumulates the diagnostics per thread and reduces them itself: one row per CTA
-    int spec_grid;
-    int64_t spec_first[3];
-    int64_t spec_cells[3];
-};
-
-static FusedGeom fused_geometry(const FusedPlan &p)
+// The one place that decides how plan p is launched over cells[g] cells from first[g] on: whole 512-cell blocks through
+// the 128-bit kernel (specialised persistent kernel or generic direct-load kernel), the ragged remainder (or everything,
+// if an array is misaligned) through the guarded kernel.  The bias slab's alignment is part of the decision; it holds for
+// every month, because corr_stride keeps each month slab 16-byte aligned.
+FusedLaunch resolve_fused(const FusedPlan &p, const int64_t first[3], const int64_t cells_in[3], int staged, int dyn_min_tiles)
 {
-    FusedGeom G;
-    memset(&G, 0, sizeof G);
-    const bool al = plan_aligned(p);
+    FusedLaunch L;
+    memset(&L, 0, sizeof L);
+    const bool al = plan_aligned(p, first);
     int nbm[3], nbt[3];
     for (int g = 0; g < 3; ++g) {
         const bool active = (g == 0) ? (p.do_early || p.do_normal) : (p.do_normal != 0);
-        const int64_t cells = active ? p.cells[g] : 0;
+        const int64_t cells = active ? cells_in[g] : 0;
         const int64_t whole = al ? (cells / kFusedCellsPerBlock) : 0;
         nbm[g] = (int)whole;
-        G.main.first[g] = p.cell0[g];
-        G.main.count[g] = whole * kFusedCellsPerBlock;
-        G.tail.first[g] = p.cell0[g] + whole * kFusedCellsPerBlock;
-        G.tail.count[g] = cells - whole * kFusedCellsPerBlock;
-        nbt[g] = (int)((G.tail.count[g] + kFusedCellsPerBlock - 1) / kFusedCellsPerBlock);
+        L.main.first[g] = first[g];
+        L.main.count[g] = whole * kFusedCellsPerBlock;
+        L.tail.first[g] = first[g] + whole * kFusedCellsPerBlock;
+        L.tail.count[g] = cells - whole * kFusedCellsPerBlock;
+        nbt[g] = (int)((L.tail.count[g] + kFusedCellsPerBlock - 1) / kFusedCellsPerBlock);
     }
-    G.main.nb_t = nbm[0];
-    G.main.nb_u = nbm[1];
-    G.nb_main = nbm[0] + nbm[1] + nbm[2];
-    G.tail.nb_t = nbt[0];
-    G.tail.nb_u = nbt[1];
-    G.nb_tail = nbt[0] + nbt[1] + nbt[2];
-    G.main.row0 = 0;
-    G.tail.row0 = (int64_t)G.nb_main * (kFusedThreads / 32);
+    L.main.nb_t = nbm[0];
+    L.main.nb_u = nbm[1];
+    L.nb_main = nbm[0] + nbm[1] + nbm[2];
+    L.tail.nb_t = nbt[0];
+    L.tail.nb_u = nbt[1];
+    L.nb_tail = nbt[0] + nbt[1] + nbt[2];
+    L.main.row0 = 0;
+    L.tail.row0 = (int64_t)L.nb_main * (kFusedThreads / 32);
+    L.diag_rows = L.tail.row0 + (int64_t)L.nb_tail * (kFusedThreads / 32);
     // specialised persistent kernel for the canonical plans with one or two surface types, whatever the grid size (20 000 cells:
-    // 6 us per step against 20 us on the generic kernels); it takes the ragged remainder along: one launch
-    G.spec = false;
-    if (al && p.S <= 2 && p.staged >= 1 && G.nb_main + G.nb_tail > 0) {
-        for (int g = 0; g < 3; ++g) {
-            G.spec_first[g] = G.main.first[g];
-            G.spec_cells[g] = G.main.count[g] + G.tail.count[g];
-        }
-        G.spec_grid = spec_applicable(p, G.spec_first, G.spec_cells);
-        if (G.spec_grid > 0) {
-            G.spec = true;
-            G.diag_accum = (p.diag != 0);
-            G.nb_main = 1;      // one launch
-            G.nb_tail = 0;
-            G.tail.nb_t = G.tail.nb_u = 0;
-            G.tail.row0 = G.spec_grid;
+    // 6 us per step against 20 us on the generic kernels); it takes the ragged remainder along: one launch, one diagnostics
+    // row per CTA
+    if (al && p.S <= 2 && staged >= 1 && L.nb_main + L.nb_tail > 0) {
+        int64_t spec_cells[3];
+        for (int g = 0; g < 3; ++g) spec_cells[g] = L.main.count[g] + L.tail.count[g];
+        if (spec_resolve(p, L.main.first, spec_cells, dyn_min_tiles, L)) {
+            L.spec = true;
+            L.diag_rows = L.spec_grid;
+            L.fills = L.spec_grid >= spec_capacity(p.S);
         }
     }
-    return G;
-}
-
-// 1: the main part of this plan runs on the specialised persistent kernel, 0: on the generic fused kernel
-int fused_uses_spec(const FusedPlan &p) { return fused_geometry(p).spec ? 1 : 0; }
-
-int fused_fills_device(const FusedPlan &p)
-{
-    const FusedGeom G = fused_geometry(p);
-    return (G.spec && G.spec_grid >= spec_capacity(p.S)) ? 1 : 0;
-}
-
-unsigned int fused_dyn_claims(const FusedPlan &p)
-{
-    const FusedGeom G = fused_geometry(p);
-    return G.spec ? spec_dyn_claims(p, G.spec_first, G.spec_cells) : 0u;
-}
-
-int64_t fused_diag_rows(const FusedPlan &p)
-{
-    const FusedGeom G = fused_geometry(p);
-    return G.tail.row0 + (int64_t)G.nb_tail * (kFusedThreads / 32);
+    return L;
 }
 
 template <int SS, int DIAG>
-static cudaError_t launch_fused_t(const FusedPlan &p, const FusedGeom &G, cudaStream_t stream, int *launches)
+static void launch_fused_t(const FusedPlan &p, const FusedLaunch &L, cudaStream_t stream, int *launches)
 {
-    if (G.nb_tail) {
-        fused_step_kernel<SS, DIAG, false><<<G.nb_tail, kFusedThreads, 0, stream>>>(p, G.tail);
+    if (L.nb_tail) {
+        fused_step_kernel<SS, DIAG, false><<<L.nb_tail, kFusedThreads, 0, stream>>>(p, L.tail);
         if (launches) *launches += 1;
     }
-    if (G.nb_main) {
-        if (G.spec) {
-            const cudaError_t e = (cudaError_t)spec_launch(p, G.spec_first, G.spec_cells, stream);
-            if (e != cudaSuccess) return e;
-        } else {
-            fused_step_kernel<SS, DIAG, true><<<G.nb_main, kFusedThreads, 0, stream>>>(p, G.main);
-        }
+    if (L.nb_main) {
+        fused_step_kernel<SS, DIAG, true><<<L.nb_main, kFusedThreads, 0, stream>>>(p, L.main);
         if (launches) *launches += 1;
     }
-    return cudaGetLastError();
 }
 
 template <int SS>
-static cudaError_t launch_fused_s(const FusedPlan &p, const FusedGeom &G, cudaStream_t stream, int *launches)
+static void launch_fused_s(const FusedPlan &p, const FusedLaunch &L, cudaStream_t stream, int *launches)
 {
-    if (p.diag >= 2) return launch_fused_t<SS, 2>(p, G, stream, launches);
-    if (p.diag == 1) return launch_fused_t<SS, 1>(p, G, stream, launches);
-    return launch_fused_t<SS, 0>(p, G, stream, launches);
+    if (p.diag >= 2) launch_fused_t<SS, 2>(p, L, stream, launches);
+    else if (p.diag == 1) launch_fused_t<SS, 1>(p, L, stream, launches);
+    else launch_fused_t<SS, 0>(p, L, stream, launches);
 }
 
-int launch_fused(const FusedPlan &p, cudaStream_t stream, int *launches)
+// one launch of a resolved plan: its parameter block with this step's fields filled in
+int launch_fused(const FusedPlan &plan, const FusedLaunch &L, const FusedStepArgs &a, cudaStream_t stream, int *launches)
 {
-    const FusedGeom G = fused_geometry(p);
-    if (G.nb_main + G.nb_tail == 0) return 0;
-    cudaError_t e;
-    switch (p.S) {
-        case 1: e = launch_fused_s<1>(p, G, stream, launches); break;
-        case 2: e = launch_fused_s<2>(p, G, stream, launches); break;
-        default: e = launch_fused_s<0>(p, G, stream, launches); break;
+    if (L.spec) {
+        SpecPlan sp = L.sp;
+        if (sp.has_bias) sp.src[0][kSpecBiasSlot] = a.bias;
+        sp.partials = a.diag_partials;
+        sp.rows = a.diag_rows;
+        sp.plane = (int64_t)plan.diag_n * a.diag_rows;
+        sp.prev = a.fold_prev;
+        sp.early_loads = a.early_loads;
+        sp.chain = sp.dyn ? 0 : a.chain;
+        sp.seq = a.chain_seq;
+        sp.done = a.chain_done;
+        sp.tile_base = a.tile_base;
+        sp.tile_counter = a.tile_counter;
+        if (const int e = spec_launch(sp, L.spec_set, L.spec_grid, stream)) return e;
+        if (launches) *launches += 1;
+        return (int)cudaGetLastError();
     }
-    return (int)e;
+    if (L.nb_main + L.nb_tail == 0) return 0;
+    FusedPlan p = plan;
+    if (p.t.bias) p.t.bias = a.bias;
+    p.diag_partials = a.diag_partials;
+    p.diag_rows = a.diag_rows;
+    switch (p.S) {
+        case 1: launch_fused_s<1>(p, L, stream, launches); break;
+        case 2: launch_fused_s<2>(p, L, stream, launches); break;
+        default: launch_fused_s<0>(p, L, stream, launches); break;
+    }
+    return (int)cudaGetLastError();
 }
 
-// partials (written by the fused launches of `p`) -> diag_out[compact slot][3]
-int launch_diag_finalize(const FusedPlan &p, double *tmp, double *diag_out, cudaStream_t stream, int *launches)
+// partials written by a generic launch of a resolved plan -> a.diag_out[compact slot][3] (a specialised launch leaves one row
+// per CTA, folded later: DiagFold)
+int launch_diag_finalize(const FusedPlan &p, const FusedLaunch &L, const FusedStepArgs &a, double *tmp, cudaStream_t stream, int *launches)
 {
     if (!p.diag || p.diag_n <= 0) return 0;
-    const FusedGeom G = fused_geometry(p);
-    if (G.spec && G.diag_accum) return 0;      // one row per CTA, folded later (DiagFold): the caller keeps track
     const int w = kFusedThreads / 32;
     DiagRanges R;
     memset(&R, 0, sizeof R);
-    const int nbm[3] = {G.main.nb_t, G.main.nb_u, G.nb_main - G.main.nb_t - G.main.nb_u};
-    const int nbt[3] = {G.tail.nb_t, G.tail.nb_u, G.nb_tail - G.tail.nb_t - G.tail.nb_u};
-    int64_t rm = 0, rt = G.tail.row0;
+    const int nbm[3] = {L.main.nb_t, L.main.nb_u, L.nb_main - L.main.nb_t - L.main.nb_u};
+    const int nbt[3] = {L.tail.nb_t, L.tail.nb_u, L.nb_tail - L.tail.nb_t - L.tail.nb_u};
+    int64_t rm = 0, rt = L.tail.row0;
     for (int g = 0; g < 3; ++g) {
         R.row_begin[g] = rm;
         rm += (int64_t)nbm[g] * w;
@@ -836,11 +803,11 @@ int launch_diag_finalize(const FusedPlan &p, double *tmp, double *diag_out, cuda
         const int g = (q == DQ_QSUR_U || q == DQ_UMOM) ? 1 : ((q == DQ_QSUR_V || q == DQ_VMOM) ? 2 : 0);
         if (p.diag_map[s] >= 0 && p.diag_map[s] < kDiagSlots) R.grid_of_slot[p.diag_map[s]] = (signed char)g;
     }
-    const int64_t rows = p.diag_rows;
+    const int64_t rows = a.diag_rows;
     const int nchunks = (int)((rows + kDiagChunk - 1) / kDiagChunk);
     const int planes = p.diag >= 2 ? 3 : 1;
-    diag_reduce_rows_kernel<<<dim3(nchunks, p.diag_n), 256, 0, stream>>>(p.diag_partials, rows, p.diag_n, planes, R, tmp, nchunks);
-    diag_reduce_final_kernel<<<p.diag_n, 256, 0, stream>>>(tmp, nchunks, planes, diag_out);
+    diag_reduce_rows_kernel<<<dim3(nchunks, p.diag_n), 256, 0, stream>>>(a.diag_partials, rows, p.diag_n, planes, R, tmp, nchunks);
+    diag_reduce_final_kernel<<<p.diag_n, 256, 0, stream>>>(tmp, nchunks, planes, a.diag_out);
     if (launches) *launches += 2;
     return (int)cudaGetLastError();
 }

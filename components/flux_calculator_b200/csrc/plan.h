@@ -7,6 +7,9 @@
 //                 outputs) because each op reads/writes global memory in the reference's order.
 //   * FusedPlan : the same work for "canonical" configurations (no aliased outputs) as ONE pass over
 //                 SoA fields with every intermediate in registers.
+// How a FusedPlan is launched over a cell range -- specialised or generic kernel, grid, schedule, diagnostics rows -- is
+// decided in one place, resolve_fused (kernels.cu, with spec_resolve in spec_kernel.cu for the specialised kernel), once
+// per prepared plan; the result is a FusedLaunch.  A step fills in its FusedStepArgs and calls launch_fused.
 #pragma once
 
 #include <stdint.h>
@@ -153,28 +156,13 @@ struct FusedPlan {
     int do_early;            // RBBR (+ its average) in this launch
     int do_normal;           // everything else
     int diag;                // accumulate diagnostics
-    int64_t cell0[3];        // first cell of this launch on each grid (chunked host pipeline)
-    int64_t cells[3];        // number of cells of this launch on each grid
     Consts c;
     FusedT t;
     FusedUV uv[2];           // [0] = u grid, [1] = v grid
-    DiagFold fold_prev;      // rows of the previous specialised launch of the stream, folded by this launch (nslots == 0: none)
-    int early_loads;         // the previous operation of the stream is this library's own step kernel (which writes no
-                             // input): the producers may start their first bulk copies before griddepcontrol.wait
-    int dyn_min_tiles;       // dynamic schedule from this many tiles per CTA on (0: the built-in default)
-    int chain;               // static schedule: the previous launch of the stream was this very plan -> its CTA b hands over to this
-    unsigned int chain_seq;  //   launch's CTA b (spec_kernel.cu); number of this launch, and where the CTAs record it
-    int pad4;
-    unsigned int *chain_done;
-    unsigned int tile_base;  // dynamic tile schedule of the specialised kernel without diagnostics: the counter's value
-    unsigned int *tile_counter;   // before this launch (it is never reset, see spec_kernel.cu)
-    double *diag_out;        // [sum|min|max][kDiagSlots] result of this step
     double *diag_partials;   // [plane: sum|min|max][diag_n][diag_rows]
     int64_t diag_rows;       // warp rows of one fused step (row stride of the partials)
     int diag_n;              // number of active diagnostics slots
     signed char diag_map[(kMaxSurfaceTypes + 1) * 10];   // slot -> compact index, -1 = inactive
-    int staged;              // specialised persistent kernel: 0 never, >= 1 whenever the plan fits
-    int pad2;
 };
 
 // diagnostics slot layout: slot(type 0..10, quantity)
@@ -187,24 +175,103 @@ constexpr int kFusedMinBlocks = 2;                           // __launch_bounds_
 constexpr int kFusedVec = 2;                                  // cells per thread (128-bit accesses)
 constexpr int kFusedCellsPerBlock = kFusedThreads * kFusedVec;
 
+// FULL = true : every thread owns V whole cells and every array is 16-byte aligned (128-bit accesses only);
+//               launched over floor(cells/V) cell vectors per grid.
+// FULL = false: guarded scalar accesses; launched over the ragged remainder (cells % V) of each grid, or over
+//               everything when a bound array is not 16-byte aligned.  first[] = first cell of this launch.
+struct LaunchGeom {
+    int nb_t, nb_u;          // blocks of the t / u grid (the rest is the v grid)
+    int64_t first[3];        // first cell handled by this launch on each grid
+    int64_t count[3];        // cells handled by this launch on each grid
+    int64_t row0;            // first diagnostics row of this launch
+};
+
+// parameter block of the specialised persistent kernel (spec_kernel.cu)
+constexpr int kSpecMaxSlots = 16;
+constexpr int kSpecMaxNS = 2;                            // surface types the specialised kernel handles
+constexpr int kSpecBiasSlot = 6;                         // src[0] slot of the bias month slab (spec_kernel.cu: Lay::BIAS)
+struct SpecPlan {
+    Consts c;
+    int64_t first[3];                 // first cell of the range on each grid
+    int64_t end[3];                   // one past its last cell
+    int ntiles[3];                    // ceil(cells / tile): the last tile of a grid may be partial (guarded path)
+    int rot[3];                       // static schedule: CTA that takes tile 0 of each grid
+    int ns;                           // number of surface types (the kernel has it as NS)
+    int t_stages, u_stages;           // the two carvings of the ring
+    int t_stage_bytes, u_stage_bytes;
+    int t_bars, u_bars;               // lcm(teams, stages): tile i uses barrier i mod bars (one per (team, stage) pair) in phase i / bars
+    int do_early;                     // RBBR in this launch
+    int has_bias, has_rsdr;
+    int any_avg_t;                    // some t-grid flux is area-fraction averaged (FARE is staged)
+    int ase_slot;                     // bulk: slot of the sensible-heat transfer coefficient (AEV for CCLM, ASE for MOM5)
+    int diag;
+    double latent_heat[kSpecMaxNS];
+    const double *src[3][kSpecMaxSlots];   // per grid: source array of each stage slot (null: slot unused)
+    uint32_t tx_bytes[3];             // bytes one tile of that grid brings in
+    const double *area[3];
+    double *out[kSpecMaxNS + 1][DQ_COUNT];   // [surface type, 0 = average][quantity] (null: not produced)
+    double *partials;                 // [plane][compact slot][row]; rows [0, grid) are this kernel's (one per CTA)
+    int64_t rows, plane;
+    DiagFold prev;                    // rows of the previous launch, folded here while the ring fills (nslots == 0: none)
+    int early_loads;                  // first bulk copies before griddepcontrol.wait (previous kernel = own step)
+    int dyn;                          // this launch uses the dynamic schedule
+    int chain;                        // static schedule: the previous launch of the stream is the same plan -> per-CTA hand-over
+    unsigned int seq;                 // number of this launch in the context's sequence of static launches
+    unsigned int *done;               // [CTA]: seq of the last launch whose CTA of that index has stored everything (null: not recorded)
+    int area_ahead;                   // fetch the cell areas one tile ahead (pays while the launch is latency bound: few tiles per CTA)
+    unsigned int tile_base;           // dynamic schedule: value of *tile_counter before this launch's first claim
+    unsigned int *tile_counter;       // dynamic schedule: tiles are claimed with atomicAdd (never reset: the host tracks the base)
+    signed char dmap[(kSpecMaxNS + 1) * DQ_COUNT];   // type * DQ_COUNT + quantity -> compact diagnostics slot (-1: inactive)
+};
+
+// A fused plan resolved for one cell range (resolve_fused): which kernel serves it, its launch geometry and schedule.
+// All of it follows from the plan, the range and the options "staged" and "dyn_min_tiles", so it is worked out once
+// per prepared plan; a step adds only its FusedStepArgs.
+struct FusedLaunch {
+    bool spec;               // the specialised persistent kernel serves the whole range in one launch
+    // generic kernel: the 128-bit kernel over whole 512-cell blocks, the guarded kernel over the ragged rest (or over
+    // everything if an array is misaligned); a launch with no blocks is skipped
+    LaunchGeom main, tail;
+    int nb_main, nb_tail;
+    // specialised kernel: its formula set (spec_kernel.cu: SpecSet), grid, and parameter block without the per-step fields
+    int spec_set, spec_grid;
+    SpecPlan sp;
+    int64_t diag_rows;       // diagnostics rows the launch writes (one per warp; one per CTA of the specialised kernel)
+    unsigned int claims;     // dynamic schedule: by how much a launch advances its tile counter (0: static schedule)
+    bool fills;              // the specialised launch occupies every CTA slot of the device
+};
+
+// what changes from one launch of a resolved plan to the next
+struct FusedStepArgs {
+    const double *bias;      // month slab of the corrections (null: the plan has none)
+    double *diag_partials;   // [plane][compact slot][diag_rows]
+    int64_t diag_rows;       // row stride of the partials
+    double *diag_out;        // [sum|min|max][kDiagSlots] result of this step
+    // specialised kernel only
+    DiagFold fold_prev;      // rows of the previous specialised launch of the stream, folded by this launch (nslots == 0: none)
+    int early_loads;         // the previous operation of the stream is this library's own step kernel (which writes no
+                             // input): the producers may start their first bulk copies before griddepcontrol.wait
+    int chain;               // static schedule: the previous launch of the stream was this very plan -> its CTA b hands over to this
+    unsigned int chain_seq;  //   launch's CTA b (spec_kernel.cu); number of this launch, and where the CTAs record it
+    unsigned int *chain_done;
+    unsigned int tile_base;  // dynamic schedule: the counter's value before this launch (it is never reset, see spec_kernel.cu)
+    unsigned int *tile_counter;
+};
+
 // launchers (kernels.cu)
 int launch_oplist(const OpList &ops, const Consts &c, int64_t n, cudaStream_t stream);
-int launch_fused(const FusedPlan &plan, cudaStream_t stream, int *launches);
-int launch_diag_finalize(const FusedPlan &plan, double *tmp, double *diag_out, cudaStream_t stream, int *launches);
+FusedLaunch resolve_fused(const FusedPlan &plan, const int64_t first[3], const int64_t cells[3], int staged, int dyn_min_tiles);
+int launch_fused(const FusedPlan &plan, const FusedLaunch &L, const FusedStepArgs &a, cudaStream_t stream, int *launches);
+int launch_diag_finalize(const FusedPlan &plan, const FusedLaunch &L, const FusedStepArgs &a, double *tmp, cudaStream_t stream, int *launches);
 int launch_diag_post(const double *diag_out, const PeerPost &post, int n_active, cudaStream_t stream);
 int launch_diag_fold(const DiagFold &fold, cudaStream_t stream);      // spec_kernel.cu: the stand-alone fold
 int launch_diag_combine(const double *chunk_out, int nchunks, double *diag_out, cudaStream_t stream);
-int64_t fused_diag_rows(const FusedPlan &plan);
-int fused_uses_spec(const FusedPlan &plan);
 int diag_tmp_doubles(int64_t rows, int nslots);
 unsigned long long read_exact_calls();
 // specialised persistent kernel (spec_kernel.cu)
-int spec_applicable(const FusedPlan &plan, const int64_t first[3], const int64_t cells[3]);
-int spec_launch(const FusedPlan &plan, const int64_t first[3], const int64_t cells[3], cudaStream_t stream);
-unsigned int spec_dyn_claims(const FusedPlan &plan, const int64_t first[3], const int64_t cells[3]);
+bool spec_resolve(const FusedPlan &plan, const int64_t first[3], const int64_t cells[3], int dyn_min_tiles, FusedLaunch &L);
+int spec_launch(const SpecPlan &sp, int set, int grid, cudaStream_t stream);
 int spec_capacity(int num_surface_types);
-int fused_fills_device(const FusedPlan &plan);      // the specialised launch of this plan occupies every CTA slot of the device
-unsigned int fused_dyn_claims(const FusedPlan &plan);      // kernels.cu: the same for a whole fused step (0: static schedule)
 unsigned long long read_spec_exact_calls();
 int launch_transpose_corrections(const double *corr_fortran, double *corr_month_major, int64_t n, int64_t stride, cudaStream_t stream);
 inline int64_t corr_stride(int64_t n) { return (n + 1) & ~int64_t(1); }      // cells between two month slabs: even, so that each slab is 16-byte aligned

@@ -70,8 +70,6 @@ struct SpecGeom {
 };
 constexpr int kSpecMaxStages = 16;
 constexpr int kSpecMaxBars = 32;                         // barriers per set: lcm(teams, stages) <= 2 * 16
-constexpr int kSpecMaxSlots = 16;
-constexpr int kSpecMaxNS = 2;                            // surface types the specialised kernel handles
 constexpr int kSpecBadCap = 16;                          // flagged tiles remembered per warp and phase; more -> all
 
 using S2 = Vd<kSpecV>;
@@ -103,40 +101,7 @@ struct Lay {
     static constexpr int NUV = (SET == SET_BULK) ? kUShared + kPer * NS : kUShared + (NS == 1 ? 0 : NS);
 };
 static_assert(Lay<SET_BULK, 2>::NT <= kSpecMaxSlots && Lay<SET_BULK, 1>::NT == 12 && Lay<SET_BULK, 1>::NUV == 6, "");
-
-struct SpecPlan {
-    Consts c;
-    int64_t first[3];                 // first cell of the range on each grid
-    int64_t end[3];                   // one past its last cell
-    int ntiles[3];                    // ceil(cells / tile): the last tile of a grid may be partial (guarded path)
-    int rot[3];                       // static schedule: CTA that takes tile 0 of each grid
-    int ns;                           // number of surface types (the kernel has it as NS)
-    int t_stages, u_stages;           // the two carvings of the ring
-    int t_stage_bytes, u_stage_bytes;
-    int t_bars, u_bars;               // lcm(teams, stages): tile i uses barrier i mod bars (one per (team, stage) pair) in phase i / bars
-    int do_early;                     // RBBR in this launch
-    int has_bias, has_rsdr;
-    int any_avg_t;                    // some t-grid flux is area-fraction averaged (FARE is staged)
-    int ase_slot;                     // bulk: slot of the sensible-heat transfer coefficient (AEV for CCLM, ASE for MOM5)
-    int diag;
-    double latent_heat[kSpecMaxNS];
-    const double *src[3][kSpecMaxSlots];   // per grid: source array of each stage slot (null: slot unused)
-    uint32_t tx_bytes[3];             // bytes one tile of that grid brings in
-    const double *area[3];
-    double *out[kSpecMaxNS + 1][DQ_COUNT];   // [surface type, 0 = average][quantity] (null: not produced)
-    double *partials;                 // [plane][compact slot][row]; rows [0, grid) are this kernel's (one per CTA)
-    int64_t rows, plane;
-    DiagFold prev;                    // rows of the previous launch, folded here while the ring fills (nslots == 0: none)
-    int early_loads;                  // first bulk copies before griddepcontrol.wait (previous kernel = own step)
-    int dyn;                          // this launch uses the dynamic schedule
-    int chain;                        // static schedule: the previous launch of the stream is the same plan -> per-CTA hand-over
-    unsigned int seq;                 // number of this launch in the context's sequence of static launches
-    unsigned int *done;               // [CTA]: seq of the last launch whose CTA of that index has stored everything (null: not recorded)
-    int area_ahead;                   // fetch the cell areas one tile ahead (pays while the launch is latency bound: few tiles per CTA)
-    unsigned int tile_base;           // dynamic schedule: value of *tile_counter before this launch's first claim
-    unsigned int *tile_counter;       // dynamic schedule: tiles are claimed with atomicAdd (never reset: the host tracks the base)
-    signed char dmap[(kSpecMaxNS + 1) * DQ_COUNT];   // type * DQ_COUNT + quantity -> compact diagnostics slot (-1: inactive)
-};
+static_assert(Lay<SET_BULK, 1>::BIAS == kSpecBiasSlot && Lay<SET_RCO, 2>::BIAS == kSpecBiasSlot, "plan.h: kSpecBiasSlot");
 
 template <int NS, int DIAG>
 struct WarpSums {    // per-CTA staging of the consumer warps' diagnostics
@@ -1460,17 +1425,6 @@ static bool spec_build(const FusedPlan &p, const int64_t first[3], const int64_t
     sp.area[1] = p.uv[0].area;
     sp.area[2] = p.uv[1].area;
     for (int k = 0; k < (kSpecMaxNS + 1) * DQ_COUNT; ++k) sp.dmap[k] = p.diag ? p.diag_map[k] : (signed char)-1;
-    sp.partials = p.diag_partials;
-    sp.rows = p.diag_rows;
-    sp.plane = (int64_t)p.diag_n * p.diag_rows;
-    sp.prev = p.fold_prev;
-    sp.tile_counter = p.tile_counter;
-    sp.tile_base = p.tile_base;
-    sp.dyn = p.dyn_min_tiles;
-    sp.chain = p.chain;
-    sp.seq = p.chain_seq;
-    sp.done = p.chain_done;
-    sp.early_loads = p.early_loads;
     *set_out = set;
     return true;
 }
@@ -1487,38 +1441,45 @@ static int spec_grid(const SpecPlan &sp)
 // CTAs of the specialised kernel the device holds at once
 int spec_capacity(int num_surface_types) { return SpecGeomCtas(num_surface_types) * spec_num_sms(); }
 
-// > 0: the plan fits the specialised kernel, value = its grid size (= diagnostics rows); 0: it does not
-int spec_applicable(const FusedPlan &p, const int64_t first[3], const int64_t cells[3])
-{
-    SpecPlan sp;
-    int set = 0;
-    if (cells[0] + cells[1] + cells[2] <= 0 || !spec_build(p, first, cells, sp, &set)) return 0;
-    return spec_grid(sp);
-}
-
-// dynamic schedule: by how much a launch of this plan advances the tile counter (every tile is claimed once, every CTA's
-// producer makes one failing claim); 0: the plan runs on the static schedule
 // tiles per CTA from which the dynamic schedule is used: below, the static one has nothing to lose to imbalance and the
 // claims would only add latency (measured, RCO set at 10^6 cells = 20 tiles per CTA: 29.2 us static, 32.7 us dynamic)
 constexpr int kSpecDynMinTiles = 48;
-static bool spec_wants_dyn(const SpecPlan &sp)
+static bool spec_wants_dyn(const SpecPlan &sp, int dyn_min_tiles)
 {
     if (sp.diag) return false;
     // Two surface types keep the static schedule unless the caller asks (option dyn_min_tiles): a t tile is 128 KB of traffic
     // and ~9 us of a team's time there, claims are coarse against 132 tiles per CTA, and consecutive static steps hand over
     // per CTA -- measured on C5 (10^7 cells, call 14, two repetitions): static 0.908 / 0.909 ms, dynamic 0.922 / 0.926 ms.
-    if (sp.ns > 1 && sp.dyn <= 0) return false;
-    const int64_t min_tiles = sp.dyn > 0 ? sp.dyn : kSpecDynMinTiles;      // (before the launch sp.dyn carries the caller's threshold)
+    if (sp.ns > 1 && dyn_min_tiles <= 0) return false;
+    const int64_t min_tiles = dyn_min_tiles > 0 ? dyn_min_tiles : kSpecDynMinTiles;
     return (int64_t)sp.ntiles[0] + sp.ntiles[1] + sp.ntiles[2] >= min_tiles * spec_grid(sp);
 }
 
-unsigned int spec_dyn_claims(const FusedPlan &p, const int64_t first[3], const int64_t cells[3])
+// the specialised half of resolve_fused (kernels.cu): if the plan fits the specialised kernel over this range, L gets the
+// kernel's parameter block without the per-step fields, its formula set, grid and schedule
+bool spec_resolve(const FusedPlan &p, const int64_t first[3], const int64_t cells[3], int dyn_min_tiles, FusedLaunch &L)
 {
-    SpecPlan sp;
+    SpecPlan &sp = L.sp;
     int set = 0;
-    if (cells[0] + cells[1] + cells[2] <= 0 || !spec_build(p, first, cells, sp, &set) || !spec_wants_dyn(sp)) return 0;
+    if (cells[0] + cells[1] + cells[2] <= 0 || !spec_build(p, first, cells, sp, &set)) return false;
+    const int grid = spec_grid(sp);
+    sp.dyn = spec_wants_dyn(sp, dyn_min_tiles) ? 1 : 0;
+    // static schedule: the three grids follow each other round the CTAs (positions b, b + G, ... of the concatenated list).
+    // (Choosing the starts so that the CTAs with one tile more spread evenly over the SMs by bytes was tried for the chained
+    // 8-GPU shards -- 2480 vs 2404 KB per SM with plain succession -- and measured no gain: 61.2 vs 60.2 us, within the
+    // box-to-box spread; profiles/README.md.)
+    sp.rot[0] = 0;
+    sp.rot[1] = grid > 0 ? sp.ntiles[0] % grid : 0;
+    sp.rot[2] = grid > 0 ? (int)(((int64_t)sp.ntiles[0] + sp.ntiles[1]) % grid) : 0;
+    // cell areas one tile ahead while there are few tiles per CTA (8-GPU shard of C4, 25 tiles per CTA: 61.3 -> 58.3 us);
+    // with many the kernel is DRAM bound and the earlier loads only synchronise the warps (10^7 cells: 0.433 -> 0.455 ms)
+    sp.area_ahead = ((int64_t)sp.ntiles[0] + sp.ntiles[1] + sp.ntiles[2] < (int64_t)64 * grid) ? 1 : 0;
+    L.spec_set = set;
+    L.spec_grid = grid;
+    // dynamic schedule: every tile is claimed once, every CTA's producer makes one failing claim
     const unsigned nuv = (unsigned)(sp.ntiles[1] + sp.ntiles[2]);
-    return (unsigned int)sp.ntiles[0] + (nuv + kDynUvBatch - 1) / kDynUvBatch + 2u * (unsigned)spec_grid(sp);
+    L.claims = sp.dyn ? (unsigned int)sp.ntiles[0] + (nuv + kDynUvBatch - 1) / kDynUvBatch + 2u * (unsigned)grid : 0u;
+    return true;
 }
 
 template <int SET, int NS, int DIAG, bool DYN>
@@ -1558,26 +1519,11 @@ static cudaError_t spec_launch_d(const SpecPlan &sp, int grid, cudaStream_t stre
     return spec_launch_t<SET, NS, 0, false>(sp, grid, stream);
 }
 
-int spec_launch(const FusedPlan &p, const int64_t first[3], const int64_t cells[3], cudaStream_t stream)
+// sp: a resolved parameter block (spec_resolve) with the per-step fields filled in
+int spec_launch(const SpecPlan &sp, int set, int grid, cudaStream_t stream)
 {
-    SpecPlan sp;
-    int set = 0;
-    if (!spec_build(p, first, cells, sp, &set)) return (int)cudaErrorInvalidValue;
     if (sp.diag && !sp.partials) return (int)cudaErrorInvalidValue;
-    const int grid = spec_grid(sp);
-    sp.dyn = spec_wants_dyn(sp) ? 1 : 0;
     if (sp.dyn && !sp.tile_counter) return (int)cudaErrorInvalidValue;
-    if (sp.dyn) sp.chain = 0;
-    // static schedule: the three grids follow each other round the CTAs (positions b, b + G, ... of the concatenated list).
-    // (Choosing the starts so that the CTAs with one tile more spread evenly over the SMs by bytes was tried for the chained
-    // 8-GPU shards -- 2480 vs 2404 KB per SM with plain succession -- and measured no gain: 61.2 vs 60.2 us, within the
-    // box-to-box spread; profiles/README.md.)
-    sp.rot[0] = 0;
-    sp.rot[1] = grid > 0 ? sp.ntiles[0] % grid : 0;
-    sp.rot[2] = grid > 0 ? (int)(((int64_t)sp.ntiles[0] + sp.ntiles[1]) % grid) : 0;
-    // cell areas one tile ahead while there are few tiles per CTA (8-GPU shard of C4, 25 tiles per CTA: 61.3 -> 58.3 us);
-    // with many the kernel is DRAM bound and the earlier loads only synchronise the warps (10^7 cells: 0.433 -> 0.455 ms)
-    sp.area_ahead = ((int64_t)sp.ntiles[0] + sp.ntiles[1] + sp.ntiles[2] < (int64_t)64 * grid) ? 1 : 0;
     cudaError_t e;
     if (set == SET_BULK) e = (sp.ns == 1) ? spec_launch_d<SET_BULK, 1>(sp, grid, stream) : spec_launch_d<SET_BULK, 2>(sp, grid, stream);
     else e = (sp.ns == 1) ? spec_launch_d<SET_RCO, 1>(sp, grid, stream) : spec_launch_d<SET_RCO, 2>(sp, grid, stream);
