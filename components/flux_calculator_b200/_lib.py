@@ -100,6 +100,7 @@ SIGNATURES = {
     "fc_set_option": (C.c_int, [ctx_p, C.c_char_p, i64]),
     "fc_get_info": (i64, [ctx_p, C.c_char_p]),
     "fc_get_diagnostics": (C.c_int, [ctx_p, C.c_int, C.c_int, C.c_int, c_double_p]),
+    "fc_get_diagnostics_history": (C.c_int, [ctx_p, C.c_int, C.c_int, C.c_int, i64, i64, c_double_p]),
     "fc_comm_get_unique_id": (C.c_int, [C.c_char_p]),
     "fc_comm_init": (C.c_int, [ctx_p, C.c_char_p, C.c_int, C.c_int]),
     "fc_configure_from_namelist": (C.c_int, [ctx_p, C.c_char_p, C.c_int]),

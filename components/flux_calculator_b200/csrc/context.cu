@@ -300,6 +300,7 @@ extern "C" int fc_destroy(fc_context *c)
     cudaFree(c->diag_chunk_out);
     cudaFree(c->tile_ctr);
     cudaFree(c->chain_done);
+    cudaFree(c->hist_ring);
     for (auto &g : c->step_graph)
         if (g) cudaGraphExecDestroy(g);
     p2p_destroy(c);
@@ -566,6 +567,40 @@ extern "C" int fc_set_time(fc_context *c, int64_t t)
     return FC_OK;
 }
 
+// the instantiated graphs of fc_run_steps; they are captured again when next needed
+static void drop_step_graphs(fc_context *c)
+{
+    for (auto &g : c->step_graph)
+        if (g) {
+            cudaGraphExecDestroy(g);
+            g = nullptr;
+        }
+}
+
+// option "diagnostics_history" = len: a new ring (none for 0) and step numbering from 0.  Whether the history is kept is
+// part of what a step graph does (captured folds of intermediate steps, addresses in the ring), so the graphs go too.
+static int set_diag_history(fc_context *c, int64_t len)
+{
+    if (len < 0 || len > ((int64_t)1 << 32)) return fail(c, FC_ERR_ARG, "fc_set_option: diagnostics_history must be in [0, 2^32]");
+    cudaSetDevice(c->device);
+    if (int rc = flush_fold(c)) return rc;
+    CUDA_TRY(c, cudaStreamSynchronize(c->stream));
+    cudaFree(c->hist_ring);
+    c->hist_ring = nullptr;
+    c->hist_base = nullptr;
+    c->hist_len = 0;
+    c->hist_steps = 0;
+    drop_step_graphs(c);
+    if (len > 0) {
+        const size_t row = (size_t)3 * kDiagSlots;
+        CUDA_TRY(c, cudaMalloc(&c->hist_ring, sizeof(double) * row * (size_t)len + sizeof(int64_t)));
+        c->hist_base = reinterpret_cast<int64_t *>(c->hist_ring + row * (size_t)len);
+        c->hist_len = len;
+    }
+    c->hist_bundle.assign((size_t)len, -1);
+    return FC_OK;
+}
+
 extern "C" int fc_set_option(fc_context *c, const char *name, int64_t value)
 {
     if (!c || !name) return fail(c, FC_ERR_ARG, "fc_set_option: NULL argument");
@@ -578,6 +613,7 @@ extern "C" int fc_set_option(fc_context *c, const char *name, int64_t value)
     else if (!strcmp(name, "chain")) c->chain_steps = value != 0;
     else if (!strcmp(name, "download")) c->download_sent_only = value != 0;
     else if (!strcmp(name, "dyn_min_tiles")) c->dyn_min_tiles = (int)std::max<int64_t>(0, std::min<int64_t>(value, 1 << 30));
+    else if (!strcmp(name, "diagnostics_history")) return set_diag_history(c, value);
     else if (!strcmp(name, "stream_touched")) {      // the caller enqueued own work on fc_get_stream(): no shortcut across it
         c->tail_own_step = false;
         return FC_OK;
@@ -1315,11 +1351,8 @@ static int prepare_impl(fc_context *c, int strict)
                 return fail(c, FC_ERR_MISSING, "diagnostics are enabled but fc_set_area was not called for the %s", kGridNames[g]);
     if (c->corr_enabled && !c->corr_dev) return fail(c, FC_ERR_STATE, "corrections enabled without data");
     for (int k = 0; k < 3; ++k) c->fused[k] = FusedBundle();
-    for (auto &g : c->step_graph)
-        if (g) {
-            cudaGraphExecDestroy(g);
-            g = nullptr;
-        }
+    c->hist_steps = 0;      // the history's rows refer to the bundles that are rebuilt here
+    drop_step_graphs(c);
     if (!c->force_generic) {
         build_fused(c, true, false, c->fused[0]);
         build_fused(c, false, true, c->fused[1]);
@@ -1430,6 +1463,7 @@ static int ensure_diag_storage(fc_context *c, const FusedPlan &P, const FusedLau
         c->diag_partials = nullptr;
         CUDA_TRY(c, cudaMalloc(&c->diag_partials, need));
         c->diag_partials_cap = need;
+        drop_step_graphs(c);      // they address the old rows
     }
     c->diag_chunk_stride = stride;
     for (int b = 0; b < 2; ++b)
@@ -1462,6 +1496,7 @@ static void diag_chunk_view(const fc_context *c, const FusedStepArgs &a, int k, 
     q.diag_partials = c->diag_partials + (size_t)k * c->diag_chunk_stride;
     q.diag_rows = a.diag_rows;
     q.diag_out = (K == 1) ? a.diag_out : c->diag_chunk_out + (size_t)k * 3 * kDiagSlots;
+    q.hist = (K == 1) ? a.hist : DiagHist{};      // K > 1: the combined vector goes to the history
 }
 
 static double *diag_tmp(const FusedPlan &P, const FusedStepArgs &a)
@@ -1491,6 +1526,7 @@ static DiagFold make_fold(const FusedPlan &P, const FusedLaunch &L, const FusedS
     f.nslots = P.diag_n;
     f.level = P.diag;
     f.out = a.diag_out;
+    f.hist = a.hist;
     return f;
 }
 
@@ -1518,6 +1554,26 @@ static void diag_step_done(fc_context *c, const FusedBundle &F)
     c->diag_level = F.plan.diag;
 }
 
+// history row of the next directly issued step (ring == null: the history is off); the step counts only once it has been
+// issued (hist_record), so a step that fails leaves no row that was never written
+static DiagHist hist_next(const fc_context *c)
+{
+    DiagHist h{};
+    if (!c->hist_len) return h;
+    h.ring = c->hist_ring;
+    h.len = c->hist_len;
+    h.step = c->hist_steps;
+    return h;
+}
+
+// n steps of bundle F, issued: the next rows of the history are theirs
+static void hist_record(fc_context *c, const FusedBundle &F, int n)
+{
+    if (!c->hist_len) return;
+    for (int s = 0; s < n; ++s) c->hist_bundle[(size_t)((c->hist_steps + s) % c->hist_len)] = (signed char)(&F - c->fused);
+    c->hist_steps += n;
+}
+
 static int ensure_tile_counters(fc_context *c)
 {
     if (!c->tile_ctr) {
@@ -1541,9 +1597,11 @@ static int attach_tile_counter(fc_context *c, const FusedLaunch &L, FusedStepArg
 // one device-resident step on the context's stream.  Which kernel runs and how it is scheduled was decided when the plan
 // was prepared (F.step, kernels.cu: resolve_fused); what is left here is this step's arguments.  gstep < 0: an ordinary
 // step.  gstep >= 0: step number gstep of a sequence that is being captured into a CUDA graph (fc_run_steps): nothing here
-// may depend on state that changes between two launches of that graph -- no fold of the previous step's rows (only the
-// last step's diagnostics are ever read; the caller registers them after the graph), one row set, tile counters that the
-// graph's leading memset node zeroes (step s uses counter s mod 2 at base (s / 2) * claims), no event records, no allocation.
+// may depend on state that changes between two launches of that graph -- tile counters that the graph's leading memset
+// node zeroes (step s uses counter s mod 2 at base (s / 2) * claims), no event records, no allocation.  Of the diagnostics
+// only the last step's vector is read unless the history is on (the caller registers it after the graph): then step s
+// folds step s - 1's rows into its history row, found through the base word the host sets before each replay, and the
+// steps alternate between two row sets by s mod 2; otherwise there is no fold in the graph and one row set.
 static int launch_resident(fc_context *c, const FusedBundle &F, const double *bias, int gstep)
 {
     const bool graph = gstep >= 0;
@@ -1564,8 +1622,18 @@ static int launch_resident(fc_context *c, const FusedBundle &F, const double *bi
         a.diag_partials = c->diag_partials;
         a.diag_rows = c->diag_rows_1;
         a.diag_out = c->diag_buf[b];
-        diag_chunk_view(c, a, graph ? 0 : (c->row_set ^= 1), 1, a);
+        if (!graph) a.hist = hist_next(c);
+        else if (c->hist_len) a.hist = DiagHist{c->hist_ring, c->hist_base, gstep, c->hist_len};
+        const bool graph_folds = graph && c->hist_len && spec;
+        diag_chunk_view(c, a, graph ? (graph_folds ? (gstep & 1) : 0) : (c->row_set ^= 1), 1, a);
         if (!graph && c->fold_pending) a.fold_prev = c->fold;
+        if (graph_folds && gstep > 0) {
+            FusedStepArgs q = a;
+            diag_chunk_view(c, a, (gstep - 1) & 1, 1, q);
+            q.diag_out = nullptr;      // an intermediate step of the graph: its vector goes to the history only
+            q.hist.step = gstep - 1;
+            a.fold_prev = make_fold(P, L, q);
+        }
     }
     a.early_loads = (spec && c->early_loads && (graph ? gstep > 0 : c->tail_own_step)) ? 1 : 0;
     // dynamic schedule: consecutive steps alternate between two counters, because the producers of a step may claim
@@ -1623,7 +1691,10 @@ static int launch_resident(fc_context *c, const FusedBundle &F, const double *bi
         } else if (int rc = finalize_chunk(c, P, L, a, c->stream)) {
             return rc;
         }
-        if (!graph) diag_step_done(c, F);
+        if (!graph) {
+            hist_record(c, F, 1);
+            diag_step_done(c, F);
+        }
     }
     if (!F.extra.empty())
         if (int rc = run_ops(c, F.extra)) return rc;
@@ -1668,8 +1739,10 @@ static int run_fused(fc_context *c, FusedBundle &F, bool async_device_only)
     FusedStepArgs a{};
     a.bias = bias;
     if (int rc = flush_fold(c)) return rc;
-    if (P.diag)
+    if (P.diag) {
         if (int rc = ensure_diag_storage(c, P, F.chunks.data(), K, a)) return rc;
+        a.hist = hist_next(c);
+    }
     c->tail_own_step = false;
     CUDA_TRY(c, cudaStreamSynchronize(c->stream));
     for (int k = 0; k < K; ++k) {
@@ -1710,9 +1783,10 @@ static int run_fused(fc_context *c, FusedBundle &F, bool async_device_only)
     for (int b : up) c->bufs[b].dev_valid = true;
     if (P.diag) {
         if (K > 1) {      // fold the chunks' result vectors in chunk order
-            if (launch_diag_combine(c->diag_chunk_out, K, a.diag_out, c->stream)) return fail(c, FC_ERR_CUDA, "diag combine launch failed");
+            if (launch_diag_combine(c->diag_chunk_out, K, a.diag_out, a.hist, c->stream)) return fail(c, FC_ERR_CUDA, "diag combine launch failed");
             c->launches += 1;
         }
+        hist_record(c, F, 1);
         diag_step_done(c, F);
     }
     if (!F.extra.empty())
@@ -1867,16 +1941,30 @@ extern "C" int fc_run_steps(fc_context *c, int64_t t0, int64_t dt, int nsteps)
         int run = 1;      // steps k .. k + run - 1 share the month
         while (k + run < nsteps && (!(F.ok && F.plan.t.bias) || fc_current_month(c->init_date, t0 + (int64_t)(k + run) * dt) == month)) ++run;
         while (graphs && run >= kGraphSteps) {
+            // the diagnostics storage as the graph was captured with it: a step of another bundle since then left its own
+            // row and set strides, from which the pending fold of the graph's last step would be built below (and if the
+            // rows had to grow, the graphs, which address the old ones, are gone)
+            if (F.plan.diag) {
+                FusedStepArgs unused{};
+                if (int rc = ensure_diag_storage(c, F.plan, &F.step, 1, unused)) return rc;
+            }
             cudaGraphExec_t &g = c->step_graph[month];
             if (!g)
                 if (int rc = capture_steps(c, F, month, kGraphSteps, &g)) return rc;
             if (int rc = flush_fold(c)) return rc;      // (a directly issued step before this graph left its rows)
+            const bool hist = c->hist_len && F.plan.diag;
+            if (hist) {      // the replay's steps are hist_steps, hist_steps + 1, ...
+                if (launch_diag_hist_base(c->hist_base, c->hist_steps, c->stream)) return fail(c, FC_ERR_CUDA, "diag history base launch failed");
+                c->launches += 1;
+            }
             CUDA_TRY(c, cudaGraphLaunch(g, c->stream));
+            if (hist) hist_record(c, F, kGraphSteps);
             c->graph_launches += 1;
             c->launches += (int64_t)kGraphSteps * (1 + (F.extra.empty() ? 0 : 1));
             k += kGraphSteps;
             run -= kGraphSteps;
-            // state as the graph leaves it: time, tile counters, the last step's diagnostics rows (set 0) not folded yet
+            // state as the graph leaves it: time, tile counters, the last step's diagnostics rows (set 0, or with the history
+            // on set 1 = (kGraphSteps - 1) mod 2) not folded yet
             c->time = t0 + (int64_t)(k - 1) * dt;
             if (F.step.claims) c->tile_base[kMaxChunks] = c->tile_base[kMaxChunks + 1] = (unsigned int)(kGraphSteps / 2) * F.step.claims;
             c->tail_own_step = F.step.spec && F.extra.empty();
@@ -1886,7 +1974,9 @@ extern "C" int fc_run_steps(fc_context *c, int64_t t0, int64_t dt, int nsteps)
                 a.diag_partials = c->diag_partials;
                 a.diag_rows = c->diag_rows_1;
                 a.diag_out = c->diag_buf[c->diag_cur ^ 1];
-                c->row_set = 0;
+                if (hist) a.hist = DiagHist{c->hist_ring, nullptr, c->hist_steps - 1, c->hist_len};
+                c->row_set = (hist && F.step.spec) ? (kGraphSteps - 1) & 1 : 0;
+                diag_chunk_view(c, a, c->row_set, 1, a);
                 if (F.step.spec) {
                     c->fold = make_fold(F.plan, F.step, a);
                     c->fold_pending = true;
@@ -1948,6 +2038,8 @@ extern "C" int64_t fc_get_info(const fc_context *c, const char *name)
     if (!c || !name) return -1;
     if (!strcmp(name, "launches")) return c->launches;
     if (!strcmp(name, "graph_launches")) return c->graph_launches;
+    if (!strcmp(name, "diagnostics_history")) return c->hist_len;
+    if (!strcmp(name, "diagnostics_history_steps")) return c->hist_steps;
     if (!strcmp(name, "exact_path_calls")) {   // threads that recomputed their cells with the IEEE routines (process-wide)
         cudaSetDevice(c->device);
         cudaStreamSynchronize(c->stream);
@@ -2034,6 +2126,45 @@ extern "C" int fc_get_diagnostics(fc_context *c, int i, int g, int idx, double o
     if (int rc = diag_fetch(c)) return rc;
     for (int j = 0; j < 3; ++j) out[j] = c->diag_host[s * 3 + j];
     if (c->diag_level < 2) out[1] = out[2] = nan("");   // min/max only at diagnostics level 2
+    return FC_OK;
+}
+
+extern "C" int fc_get_diagnostics_history(fc_context *c, int i, int g, int idx, int64_t first, int64_t count, double *out)
+{
+    if (!c || (!out && count > 0)) return fail(c, FC_ERR_ARG, "fc_get_diagnostics_history: NULL argument");
+    const int s = (i >= 0 && i <= FC_MAX_SURFACE_TYPES) ? diag_slot_for(i, g, idx) : -1;
+    if (s < 0) return fail(c, FC_ERR_ARG, "fc_get_diagnostics_history: no diagnostics slot for this field");
+    if (!c->hist_len) return fail(c, FC_ERR_STATE, "fc_get_diagnostics_history: no history kept: set option 'diagnostics_history'");
+    bool any = false;
+    for (const FusedBundle &F : c->fused) any = any || (F.ok && F.plan.diag && F.plan.diag_map[s] >= 0);
+    if (!any) return fail(c, FC_ERR_STATE, "fc_get_diagnostics_history: %s of surface_type %d is computed by no step with diagnostics", kVarNames[idx], i);
+    const int64_t lo = std::max<int64_t>(0, c->hist_steps - c->hist_len);
+    if (count < 0 || first < lo || first > c->hist_steps - count)
+        return fail(c, FC_ERR_ARG, "fc_get_diagnostics_history: steps [%lld, %lld) requested, steps [%lld, %lld) are retained",
+                    (long long)first, (long long)(first + count), (long long)lo, (long long)c->hist_steps);
+    cudaSetDevice(c->device);
+    if (int rc = flush_fold(c)) return rc;
+    const size_t row = (size_t)3 * kDiagSlots;
+    std::vector<double> rows((size_t)count * row);
+    for (int64_t j = 0; j < count;) {      // at most two contiguous pieces of the ring
+        const int64_t r = (first + j) % c->hist_len, n = std::min(count - j, c->hist_len - r);
+        CUDA_TRY(c, cudaMemcpyAsync(rows.data() + (size_t)j * row, c->hist_ring + (size_t)r * row, sizeof(double) * row * (size_t)n,
+                                    cudaMemcpyDeviceToHost, c->stream));
+        j += n;
+    }
+    CUDA_TRY(c, cudaStreamSynchronize(c->stream));
+    for (int64_t j = 0; j < count; ++j) {
+        const FusedPlan &P = c->fused[c->hist_bundle[(size_t)((first + j) % c->hist_len)]].plan;
+        const int k = P.diag_map[s];
+        const double *h = rows.data() + (size_t)j * row;
+        for (int q = 0; q < 3; ++q) out[3 * j + q] = nan("");
+        if (k < 0) continue;      // this step did not compute the field
+        out[3 * j] = h[k];
+        if (P.diag >= 2) {
+            out[3 * j + 1] = h[kDiagSlots + k];
+            out[3 * j + 2] = h[2 * kDiagSlots + k];
+        }
+    }
     return FC_OK;
 }
 

@@ -186,6 +186,14 @@ struct fc_context {
     std::vector<int> diag_active;        // slot ids in compact order (of the last step)
     bool diag_valid = false;
     int diag_level = 0;                  // level of the last step
+    // option "diagnostics_history" = hist_len: the result vector of each of the last hist_len steps with diagnostics, step k
+    // (counted from the last reset) in row k mod hist_len of hist_ring [hist_len][sum|min|max][kDiagSlots] (compact slots
+    // of the bundle that ran it: hist_bundle[row], 0 early, 1 normal, 2 all); hist_base = first step of the next graph replay
+    int64_t hist_len = 0;
+    int64_t hist_steps = 0;
+    double *hist_ring = nullptr;
+    int64_t *hist_base = nullptr;
+    std::vector<signed char> hist_bundle;
 
     // NCCL
     void *nccl_comm = nullptr;

@@ -540,7 +540,8 @@ diag_reduce_rows_kernel(const double *__restrict__ part, int64_t rows, int nslot
 }
 
 __global__ void __launch_bounds__(256)
-diag_reduce_final_kernel(const double *__restrict__ tmp, int nchunks, int planes, double *__restrict__ out)
+diag_reduce_final_kernel(const double *__restrict__ tmp, int nchunks, int planes, double *__restrict__ out,
+                         const __grid_constant__ DiagHist hist)
 {
     const int slot = blockIdx.x;
     double s = 0.0, mn = DBL_MAX, mx = -DBL_MAX;
@@ -559,6 +560,12 @@ diag_reduce_final_kernel(const double *__restrict__ tmp, int nchunks, int planes
         out[0 * kDiagSlots + slot] = s;
         out[1 * kDiagSlots + slot] = mn;
         out[2 * kDiagSlots + slot] = mx;
+        if (hist.ring) {
+            double *h = diag_hist_row(hist);
+            h[0 * kDiagSlots + slot] = s;
+            h[1 * kDiagSlots + slot] = mn;
+            h[2 * kDiagSlots + slot] = mx;
+        }
     }
 }
 
@@ -807,13 +814,14 @@ int launch_diag_finalize(const FusedPlan &p, const FusedLaunch &L, const FusedSt
     const int nchunks = (int)((rows + kDiagChunk - 1) / kDiagChunk);
     const int planes = p.diag >= 2 ? 3 : 1;
     diag_reduce_rows_kernel<<<dim3(nchunks, p.diag_n), 256, 0, stream>>>(a.diag_partials, rows, p.diag_n, planes, R, tmp, nchunks);
-    diag_reduce_final_kernel<<<p.diag_n, 256, 0, stream>>>(tmp, nchunks, planes, a.diag_out);
+    diag_reduce_final_kernel<<<p.diag_n, 256, 0, stream>>>(tmp, nchunks, planes, a.diag_out, a.hist);
     if (launches) *launches += 2;
     return (int)cudaGetLastError();
 }
 
 // result vectors [sum|min|max][kDiagSlots] of the chunks of one step -> one vector, in chunk order
-__global__ void diag_combine_kernel(const double *__restrict__ chunk_out, int nchunks, double *__restrict__ out)
+__global__ void diag_combine_kernel(const double *__restrict__ chunk_out, int nchunks, double *__restrict__ out,
+                                    const __grid_constant__ DiagHist hist)
 {
     const int t = threadIdx.x;
     if (t >= kDiagSlots) return;
@@ -827,6 +835,12 @@ __global__ void diag_combine_kernel(const double *__restrict__ chunk_out, int nc
     out[t] = s;
     out[kDiagSlots + t] = mn;
     out[2 * kDiagSlots + t] = mx;
+    if (hist.ring) {
+        double *h = diag_hist_row(hist);
+        h[t] = s;
+        h[kDiagSlots + t] = mn;
+        h[2 * kDiagSlots + t] = mx;
+    }
 }
 
 // peer exchange of a finished result vector (generic kernel / chunked host pipeline; the specialised kernel does it itself)
@@ -851,9 +865,18 @@ int launch_diag_post(const double *diag_out, const PeerPost &post, int n_active,
     return (int)cudaGetLastError();
 }
 
-int launch_diag_combine(const double *chunk_out, int nchunks, double *diag_out, cudaStream_t stream)
+int launch_diag_combine(const double *chunk_out, int nchunks, double *diag_out, const DiagHist &hist, cudaStream_t stream)
 {
-    diag_combine_kernel<<<1, 128, 0, stream>>>(chunk_out, nchunks, diag_out);
+    diag_combine_kernel<<<1, 128, 0, stream>>>(chunk_out, nchunks, diag_out, hist);
+    return (int)cudaGetLastError();
+}
+
+// number of the first step of the graph that is replayed next (DiagHist::base), in stream order before the replay
+__global__ void diag_hist_base_kernel(int64_t *word, int64_t base) { *word = base; }
+
+int launch_diag_hist_base(int64_t *word, int64_t base, cudaStream_t stream)
+{
+    diag_hist_base_kernel<<<1, 1, 0, stream>>>(word, base);
     return (int)cudaGetLastError();
 }
 

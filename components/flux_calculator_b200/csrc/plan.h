@@ -137,6 +137,21 @@ struct PeerPost {
     DiagMail *mail[kMaxPeers];       // mailbox base of every rank (the own one included), mapped into this process
 };
 
+// Where a step's result vector is also kept (option "diagnostics_history" = len): row step mod len of a ring
+// [len][sum|min|max][kDiagSlots].  A directly issued step knows its number; a launch inside a captured graph knows only
+// its offset within the graph, and the graph's first step number is read from *base, which the host sets before
+// every replay.
+struct DiagHist {
+    double *ring;                    // null: no history
+    const int64_t *base;             // null: step is the absolute step number
+    int64_t step, len;
+};
+__device__ __forceinline__ double *diag_hist_row(const DiagHist &h)
+{
+    const int64_t k = h.step + (h.base ? *h.base : 0);
+    return h.ring + (k % h.len) * (3 * kDiagSlotsFwd);
+}
+
 // Rows of a specialised launch (one per CTA) that still have to be folded into that step's result vector.  The
 // specialised kernel does not fold its own rows: the CTAs just leave their row and exit, and the fold runs where it
 // costs nothing -- in the producer warps of the NEXT step's kernel while its ring fills (griddepcontrol.wait orders
@@ -147,8 +162,9 @@ struct DiagFold {
     int64_t row_stride, plane;       // plane = nslots * row_stride
     int nrows, nslots;               // rows written per slot (= grid of that launch); nslots == 0: nothing to fold
     int level, pad;                  // 1: sums, 2: sums + min/max
-    double *out;                     // [sum|min|max][kDiagSlots]
+    double *out;                     // [sum|min|max][kDiagSlots] (null: only the history row, an intermediate step of a graph)
     PeerPost post;                   // nranks > 1: also post the result to every rank's mailbox
+    DiagHist hist;                   // history row of the step that wrote the rows
 };
 
 struct FusedPlan {
@@ -247,6 +263,7 @@ struct FusedStepArgs {
     double *diag_partials;   // [plane][compact slot][diag_rows]
     int64_t diag_rows;       // row stride of the partials
     double *diag_out;        // [sum|min|max][kDiagSlots] result of this step
+    DiagHist hist;           // ... and its row of the diagnostics history (ring == null: none)
     // specialised kernel only
     DiagFold fold_prev;      // rows of the previous specialised launch of the stream, folded by this launch (nslots == 0: none)
     int early_loads;         // the previous operation of the stream is this library's own step kernel (which writes no
@@ -265,7 +282,8 @@ int launch_fused(const FusedPlan &plan, const FusedLaunch &L, const FusedStepArg
 int launch_diag_finalize(const FusedPlan &plan, const FusedLaunch &L, const FusedStepArgs &a, double *tmp, cudaStream_t stream, int *launches);
 int launch_diag_post(const double *diag_out, const PeerPost &post, int n_active, cudaStream_t stream);
 int launch_diag_fold(const DiagFold &fold, cudaStream_t stream);      // spec_kernel.cu: the stand-alone fold
-int launch_diag_combine(const double *chunk_out, int nchunks, double *diag_out, cudaStream_t stream);
+int launch_diag_combine(const double *chunk_out, int nchunks, double *diag_out, const DiagHist &hist, cudaStream_t stream);
+int launch_diag_hist_base(int64_t *word, int64_t base, cudaStream_t stream);
 int diag_tmp_doubles(int64_t rows, int nslots);
 unsigned long long read_exact_calls();
 // specialised persistent kernel (spec_kernel.cu)

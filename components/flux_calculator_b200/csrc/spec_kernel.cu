@@ -385,8 +385,9 @@ __device__ __forceinline__ void consumer_barrier()
     asm volatile("bar.sync 1, %0;" ::"n"(SpecGeom<NS>::kConsumers) : "memory");
 }
 
-// one warp folds the rows of compact slot cs into the result vector: lane-strided rows, then a tree -- a fixed order, the
-// same in the next step's kernel and in the stand-alone fold kernel -- and posts the result to the peers' mailboxes
+// one warp folds the rows of compact slot cs into the result vector (and the step's history row): lane-strided rows, then
+// a tree -- a fixed order, the same in the next step's kernel and in the stand-alone fold kernel -- and posts the result
+// to the peers' mailboxes
 __device__ __forceinline__ void diag_fold_slot(const DiagFold &f, int cs)
 {
     const int lane = threadIdx.x & 31;
@@ -419,10 +420,16 @@ __device__ __forceinline__ void diag_fold_slot(const DiagFold &f, int cs)
     s = __shfl_sync(0xffffffffu, s, 0);
     mn = __shfl_sync(0xffffffffu, mn, 0);
     mx = __shfl_sync(0xffffffffu, mx, 0);
-    if (lane == 0) {
+    if (lane == 0 && f.out) {
         f.out[0 * kDiagSlots + cs] = s;
         f.out[1 * kDiagSlots + cs] = mn;
         f.out[2 * kDiagSlots + cs] = mx;
+    }
+    if (lane == 0 && f.hist.ring) {
+        double *h = diag_hist_row(f.hist);
+        h[0 * kDiagSlots + cs] = s;
+        h[1 * kDiagSlots + cs] = mn;
+        h[2 * kDiagSlots + cs] = mx;
     }
     // compute -> exchange without a collective launch: the result goes straight into every rank's mailbox over NVLink
     // as self-validating 8-byte words (no fence, no flag store: see DiagMail); one lane per (rank, plane)

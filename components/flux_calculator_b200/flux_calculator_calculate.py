@@ -185,6 +185,20 @@ class FluxCalculator:
         self._check(lib.fc_get_diagnostics(self._ctx, surface_type, grid, var_index(var), out))
         return tuple(out)
 
+    def diagnostics_history(self, surface_type, grid, var, first=None, count=None):
+        """(count, 3) float64 array: row j = diagnostics(surface_type, grid, var) as it was right after step first + j
+        (NaN where that step did not compute the field); needs option "diagnostics_history" > 0.  Default: every
+        retained step; with only count given, the last count steps."""
+        total = self.info("diagnostics_history_steps")
+        if first is None:
+            first = max(0, total - self.info("diagnostics_history")) if count is None else total - count
+        if count is None:
+            count = total - first
+        out = np.empty((max(int(count), 0), 3), dtype=np.float64)
+        self._check(lib.fc_get_diagnostics_history(self._ctx, surface_type, grid, var_index(var), int(first), int(count),
+                                                   out.ctypes.data_as(C.POINTER(C.c_double))))
+        return out
+
     def comm_init(self, unique_id, rank, nranks):
         self._check(lib.fc_comm_init(self._ctx, unique_id, rank, nranks))
 

@@ -144,6 +144,14 @@ module fluxcalc_c_api
       integer(c_int), value :: surface_type, grid, var_idx
       real(c_double), intent(out) :: out(3)
     end function
+    integer(c_int) function fc_get_diagnostics_history(ctx, surface_type, grid, var_idx, first_step, count, out) &
+        bind(c, name='fc_get_diagnostics_history')
+      import :: c_ptr, c_int, c_int64_t, c_double
+      type(c_ptr), value :: ctx
+      integer(c_int), value :: surface_type, grid, var_idx
+      integer(c_int64_t), value :: first_step, count
+      real(c_double), intent(out) :: out(3, *)      ! out(:, j + 1) = sum, min, max after step first_step + j
+    end function
     integer(c_int) function fc_comm_get_unique_id(id) bind(c, name='fc_comm_get_unique_id')
       import :: c_int, c_char
       character(kind=c_char), intent(out) :: id(128)

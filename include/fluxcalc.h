@@ -264,7 +264,8 @@ int fc_step_all(fc_context *ctx, int64_t current_step_time);
  * only) -- the time loop of flux_calculator.F90:859-1028 for a host that keeps its fields on the device.  The steps of one
  * calendar month differ in nothing (the month selects the bias slab, calculate.F90:66-73): they are issued as replays of
  * one CUDA graph of 32 step launches per month, the remainder directly.  Results are bit-identical to nsteps calls of
- * fc_step_all.  With diagnostics only the LAST step's values can be read afterwards. */
+ * fc_step_all.  With diagnostics fc_get_diagnostics reads the LAST step's values afterwards; with option
+ * "diagnostics_history" = H every step's vector is kept and fc_get_diagnostics_history reads those of the last H steps. */
 int fc_run_steps(fc_context *ctx, int64_t t0, int64_t timestep, int nsteps);
 
 int fc_synchronize(fc_context *ctx);
@@ -287,13 +288,15 @@ int fc_kernel_time_ms(fc_context *ctx, double *total_ms, int64_t *count);
  *          "force_generic" (0/1: use the op-list interpreter kernels instead of the fused kernel),
  *          "pin_host" (0/1: cudaHostRegister bound host arrays), "h2d_chunks" (pipeline depth of the
  *          host-pointer path), "diagnostics" (0 off, 1 area-weighted sums, 2 sums + min/max),
+ *          "diagnostics_history" (0 off, H: keep the diagnostics of the last H steps, fc_get_diagnostics_history),
  *          "profile_kernel" (0 off, n: time every n-th fused launch), "staged" (specialised persistent kernel: 0 never,
  *          >= 1 (default) whenever the plan fits) */
 int fc_set_option(fc_context *ctx, const char *name, int64_t value);
 int64_t fc_get_info(const fc_context *ctx, const char *name);
 /* info names: "launches" (kernel launches issued so far), "fused" (1 if the fused kernel serves
  * fc_step_*), "bytes_per_cell" (algorithmic bytes of fc_step_all per t/u/v cell triple),
- * "h2d_bytes_per_step", "d2h_bytes_per_step", "exact_path_calls" (threads of the specialised kernel / warps of the generic
+ * "h2d_bytes_per_step", "d2h_bytes_per_step", "diagnostics_history" (its length H),
+ * "diagnostics_history_steps" (steps recorded in the diagnostics history since its last reset), "exact_path_calls" (threads of the specialised kernel / warps of the generic
  * fused kernel that left the lock-step fast path and recomputed their cells with the IEEE routines; 0 for physical data) */
 
 /* ------------------------------------------------------------------------------------------------
@@ -306,6 +309,19 @@ int64_t fc_get_info(const fc_context *ctx, const char *name);
  * summation tree, i.e. on the kernel that served the step and, in host-pointer mode, on the pipeline depth
  * ("h2d_chunks": one partial vector per chunk, combined in chunk order) -- min and max do not. */
 int fc_get_diagnostics(fc_context *ctx, int surface_type, int grid, int var_idx, double out[3]);
+/* Per-step history (option "diagnostics_history" = H > 0; default 0 = off): the context keeps the result vector of each
+ * of the last H steps that ran with diagnostics.  A step is one call of fc_step_early / fc_step_normal / fc_step_all or
+ * one step of fc_run_steps; steps are numbered 0, 1, 2, ... from the last reset, which happens when the option is set
+ * and when the plan is rebuilt (fc_prepare, explicit or implicit).  fc_get_info(ctx, "diagnostics_history_steps") is
+ * the number of steps recorded since then; steps [max(0, total - H), total) are retained.
+ * out[3*j + 0..2] = what fc_get_diagnostics would have returned right after step first_step + j (sum, min, max; min and
+ * max NaN at level 1); all three are NaN if that step did not compute the field (e.g. HSEN in an fc_step_early step).
+ * The values are this rank's LOCAL values, also after fc_comm_init / fc_comm_p2p_connect (fc_allreduce_diagnostics acts
+ * on the last step only).  Waits for the context's stream.  FC_ERR_STATE: the history is off, or no step of the
+ * current plan computes the field; FC_ERR_ARG: no diagnostics slot for the field, or the window
+ * [first_step, first_step + count) reaches outside the retained steps. */
+int fc_get_diagnostics_history(fc_context *ctx, int surface_type, int grid, int var_idx, int64_t first_step,
+                               int64_t count, double *out /* count x 3, host */);
 
 #define FC_UNIQUE_ID_BYTES 128
 int fc_comm_get_unique_id(char id[FC_UNIQUE_ID_BYTES]);                  /* ncclGetUniqueId */
